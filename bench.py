@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (libcudampc.so)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path, restated (oracle/), all host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/<name>.npy
 
 Headline (`value`, `e2e`, `roofline`): BASELINE.json configs[2] - 65,536 independent horizon-50 tracking QPs with the
 steering-rate limit +-0.02 rad/step PER GPU; a "step" is one pass of the hot path over that batch.  Under torchrun every rank
@@ -29,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only; nothing is cached in it
 
 METRIC = "MPC QP solves/sec (horizon 50, batched)"
 UNIT = "solves/s"
@@ -70,6 +72,26 @@ def flops_of_batch(N, iters, n_fac, n_solves):
 def io_bytes(N, B):
     """algorithmic bytes per solve (SURVEY §8d): in 32N+80, out 48N+56."""
     return B * (32 * N + 80), B * (48 * N + 56)
+
+
+DUMP_BYTES = 60_000_000     # --dump-outputs stays under 64 MB: a fixed sample of the problems when the whole batch does not fit
+DUMP_FIELDS = ("u0", "Xp", "Up", "status", "iters", "pri_res", "dua_res", "info")
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """Every array of the BatchResult the timed path returns, as float64 (the int32 counters are exact in it), so that two builds
+    can be compared output for output.  All problems when they fit DUMP_BYTES, else the same seeded sample of problems from every
+    array; `problem_index.npy` holds the sampled problems' positions in the batch."""
+    import torch
+    B = res.u0.shape[0]
+    row_bytes = 8 * (1 + sum(int(np.prod(getattr(res, k).shape[1:])) for k in DUMP_FIELDS))
+    n = min(B, DUMP_BYTES // row_bytes)
+    idx = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    sel = torch.as_tensor(idx, device=res.u0.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "problem_index.npy"), idx.astype(np.float64))
+    for k in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f"{k}.npy"), getattr(res, k)[sel].double().cpu().numpy())
 
 
 def shard_range(rank: int, world: int, total: int):
@@ -324,7 +346,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--latency-launches", type=int, default=100, help="launches of one resident wave for the latency percentiles")
     ap.add_argument("--skip-configs", action="store_true", help="headline only: skip the config2 / config4 / config5 blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -541,6 +566,8 @@ def main():
         "cpu_baseline": cb,
         "wall_s_timed_region": max(m["wall_s"] for m in allm),
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)            # res: the last timed step of the headline
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
