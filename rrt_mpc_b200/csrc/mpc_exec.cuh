@@ -147,6 +147,80 @@ __device__ __forceinline__ void oe_backward_lanes(int lane, const View& w, const
   __syncwarp();
 }
 
+// Sequential half of the ADMM factorisation (mpc_oe.h oe_factor_half) in the same row lanes: at step i, lane r of a half
+// forms row r of G_{i+1} = F_{i+1} S'_i^-1 and row r of the update G_{i+1} F_{i+1}' of S'_{i+1} (no lane needs another lane's
+// row of G).  Every lane of the half inverts the 6x6 pivot itself with spd6_inverse, and every entry is formed by the
+// statements of oe_factor_half, so the factor is bit-identical to the one-lane version.  The two halves can differ by one
+// step: a warp barrier covers the lanes whose half has step i.  The middle stage (oe_factor_middle) stays on one lane.
+__device__ __forceinline__ void oe_factor_lanes(int lane, const View& w, const OEView& oe) {
+  if (lane < 12) {
+    const bool bottom = lane >= 6;
+    const int r = bottom ? lane - 6 : lane;
+    const OEHalf h = oe_half(w, oe, bottom);
+    double u[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};                   // row r of the middle's update U (entries c <= r)
+#pragma unroll 1
+    for (int i = 0; i < h.cnt; ++i) {
+      const unsigned mask = (i < oe.jm ? 0x3fu : 0u) | (i < oe.nb ? 0xfc0u : 0u);
+      double* sp = h.s0 + h.sstep * i;
+      double S[6][6], sv[OE_SYM];
+      sym_load(sp, sv);
+      sym_expand(sv, S);
+      spd6_inverse(S, sv);
+      sym_expand(sv, S);                                           // S = S'_i^-1 (full)
+      double* g = h.g0 + OE_G * i;                                 // block of step i+1
+      double F[OE_G], Fr[6], G[6];
+      blk_load(g, F);
+      row_load(g + 6 * r, Fr);
+      __syncwarp(mask);                                            // S'_i and F read by the whole half before they are overwritten
+      if (r == 0) {
+#pragma unroll
+        for (int t = 0; t < OE_SYM; ++t) sp[t] = sv[t];
+      }
+#pragma unroll
+      for (int c = 0; c < 6; ++c) {
+        double acc = Fr[0] * S[0][c];
+#pragma unroll
+        for (int t = 1; t < 6; ++t) acc = fma(Fr[t], S[t][c], acc);
+        G[c] = acc;
+      }
+      row_store(g + 6 * r, G);
+      double* sn = h.s0 + h.sstep * (i + 1) + MPC_SP(r, 0);         // row r of S'_{i+1}
+      const bool last = (i + 1 == h.cnt);
+#pragma unroll
+      for (int c = 0; c < 6; ++c) {
+        if (c > r) break;
+        double acc = G[0] * F[6 * c];
+#pragma unroll
+        for (int t = 1; t < 6; ++t) acc = fma(G[t], F[6 * c + t], acc);
+        if (last) u[c] = acc; else sn[c] -= acc;
+      }
+      __syncwarp(mask);                                            // S'_{i+1} complete
+    }
+    // middle stage: S'_m = S_m - U_top - U_bot (row r by lane r), then inverted by lane 0
+    double uo[6];
+#pragma unroll
+    for (int c = 0; c < 6; ++c) uo[c] = __shfl_sync(MPC_ROW_LANES, u[c], bottom ? lane : lane + 6);
+    double* sm = oe.sinv + OE_SYM * oe.jm;
+    if (!bottom) {
+#pragma unroll
+      for (int c = 0; c < 6; ++c) {
+        if (c > r) break;
+        sm[MPC_SP(r, c)] -= u[c] + uo[c];
+      }
+    }
+    __syncwarp(MPC_ROW_LANES);
+    if (lane == 0) {
+      double S[6][6], sv[OE_SYM];
+      sym_load(sm, sv);
+      sym_expand(sv, S);
+      spd6_inverse(S, sv);
+#pragma unroll
+      for (int t = 0; t < OE_SYM; ++t) sm[t] = sv[t];
+    }
+  }
+  __syncwarp();
+}
+
 __device__ __forceinline__ int next_problem_warp(int* counter, int lane) {
   int p = 0;
   if (lane == 0) p = atomicAdd(counter, 1);
@@ -323,16 +397,7 @@ struct GroupExec {
   __device__ __forceinline__ void oe_factor(const View& w, const Params& p, const Mode& m, const OEView& oe) {
     stages_par(w.N + 1, 1, [&](int k) { oe_factor_odd(w, p, m, oe, k); });
     stages_par(w.N + 1, 0, [&](int k) { oe_factor_even(w, p, m, oe, k); });
-    if (chain_warp()) {
-      double U[21], Uo[21];
-#pragma unroll
-      for (int t = 0; t < 21; ++t) U[t] = 0.0;
-      if (lane < 2) oe_factor_half(oe_half(w, oe, lane == 1), U);
-      __syncwarp();
-#pragma unroll
-      for (int t = 0; t < 21; ++t) Uo[t] = __shfl_sync(0xffffffffu, U[t], 1);
-      if (lane == 0) oe_factor_middle(oe, U, Uo);
-    }
+    if (chain_warp()) oe_factor_lanes(lane, w, oe);
     group_sync();
   }
   __device__ __forceinline__ void oe_forward(const View& w, const OEView& oe) {

@@ -58,7 +58,8 @@ __global__ void __launch_bounds__(MAXT, 1) mpc_solve_kernel(Params p, Settings s
 
 // ------------------------------------------------------------------------------------------------
 // K_solve, register form (mpc_reg.h, mpc_drv.h): two warps per problem; the iteration blocks are inlined HERE, at the top
-// level of the kernel, and everything else of the driver runs in three real calls that keep their state in shared memory.
+// level of the kernel, and everything else of the driver runs in three inlined pieces that keep their state in shared memory
+// (the after-block piece also runs once per polish pass, without a block before it).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ ProblemIO batch_io(const BatchArgs& a, int b, int N, int group) {
   const int ws = warm_size(N);
@@ -106,7 +107,7 @@ __device__ __forceinline__ void reg_drv_after(RegCtx c, int b) {
   Drv d = c.sh->drv;
   ex.group_sync();                          // every lane has its copy before lane 0 writes the new one
   drv_after(ex, w, *c.p, *c.s, io, d);
-  if (!d.finished) drv_prepare(ex, w, *c.p, *c.s, d);
+  if (!d.finished && d.phase == PH_ADMM) drv_prepare(ex, w, *c.p, *c.s, d);
   if (ex.gl() == 0) c.sh->drv = d;
   ex.group_sync();
 }
@@ -141,8 +142,10 @@ __global__ void __launch_bounds__(MAXT, 1) mpc_solve_reg_kernel(const __grid_con
     const RegCtx c{&p, &s, &a, base, sh, N, fpad, xpad, lane, warp, (int)blockIdx.x * P + warp / WPP};
     reg_drv_begin<WPP>(c, b);
     while (!*(volatile int*)&sh->drv.finished) {
-      const int nb = *(volatile int*)&sh->drv.nb;
-      reg_block_run<STATE, WPP>(base, N, fpad, xpad, p.dt, &sh->drv.ic, nb, lane, ev, bar_id, tg);
+      if (*(volatile int*)&sh->drv.phase == PH_ADMM) {       // else a polish pass ran its solves: its residuals are next
+        const int nb = *(volatile int*)&sh->drv.nb;
+        reg_block_run<STATE, WPP>(base, N, fpad, xpad, p.dt, &sh->drv.ic, nb, lane, ev, bar_id, tg);
+      }
       reg_drv_after<WPP>(c, b);
     }
     reg_drv_finish<WPP>(c, b);

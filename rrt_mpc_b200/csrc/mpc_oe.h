@@ -272,6 +272,7 @@ MPC_HD void sym_expand(const double* a, double (*A)[6]) {
 }
 // Sequential block LDL' of one half: for i = 0..cnt-1: S'_i^-1; G_{i+1} = F_{i+1} S'_i^-1; S'_{i+1} -= G_{i+1} F_{i+1}'.
 // The last update belongs to the middle stage: it is returned in U (packed lower triangle), not applied.
+// Sequential statement (host emulation); the kernel runs mpc_exec.cuh oe_factor_lanes, the same statements with one lane per row.
 MPC_HD void oe_factor_half(const OEHalf& h, double* U) {
 #pragma unroll
   for (int i = 0; i < 21; ++i) U[i] = 0.0;

@@ -1,11 +1,15 @@
-"""Static SASS instruction count of a kernel by source function (dev tool): python tools/code_size.py <kernel substring>"""
+"""Static SASS instruction count of a kernel by source function (dev tool): python tools/code_size.py <kernel substring> [binary]
+
+binary: the library (default rrt_mpc_b200/libcudampc.so) or one translation unit's object, e.g. rrt_mpc_b200/_obj/tu7.o for the
+register-form kernel (the library's kernel cubins share one name, so only the last one extracted from it is seen)."""
 import re, subprocess, sys, os, tempfile, collections, bisect
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-so = os.path.join(ROOT, "rrt_mpc_b200", "libcudampc.so"); kern = sys.argv[1]
+so = os.path.abspath(sys.argv[2]) if len(sys.argv) > 2 else os.path.join(ROOT, "rrt_mpc_b200", "libcudampc.so"); kern = sys.argv[1]
 tmp = tempfile.mkdtemp()
 subprocess.run(["cuobjdump", "-xelf", "all", so], cwd=tmp, check=True, capture_output=True)
-cub = [f for f in os.listdir(tmp) if f.endswith(".cubin")][0]
-dis = subprocess.run(["nvdisasm", "-g", "-c", os.path.join(tmp, cub)], capture_output=True, text=True).stdout.splitlines()
+dis = []                       # every cubin of the library (one per translation unit)
+for cub in sorted(f for f in os.listdir(tmp) if f.endswith(".cubin")):
+    dis += subprocess.run(["nvdisasm", "-g", "-c", os.path.join(tmp, cub)], capture_output=True, text=True).stdout.splitlines()
 csrc = os.path.join(ROOT, "rrt_mpc_b200", "csrc"); fmap = {}
 for fn in os.listdir(csrc):
     st = []
