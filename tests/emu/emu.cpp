@@ -6,6 +6,7 @@
 #include <string.h>
 #include <vector>
 #include "../../rrt_mpc_b200/csrc/mpc_solve.h"
+#include "la_systems.h"
 
 using namespace mpc;
 
@@ -64,31 +65,7 @@ extern "C" {
 int emu_footprint(int N) { return footprint(N); }
 int emu_warm_size(int N) { return warm_size(N); }
 
-// params/settings passed as flat double arrays to keep the ctypes side trivial
-//  par: L, dt, (Q+Q')[16], (R+R')[4], (QN+QN')[16], u_lo[2], u_hi[2], v_lo, v_hi, du_lo[2], du_hi[2], w_v, w_u, w_du   (51)
-//  set: eps_abs, eps_rel, rho0, alpha, sigma, adaptive_rho_tolerance, rho_eq_factor, rho_min, rho_max, delta,
-//       max_iter, check_termination, adaptive_rho, adaptive_rho_interval, polish_passes, polish_refine_iter, warm_start, polish_retry (18)
-static void unpack(const double* par, const double* set, int N, Params& p, Settings& s) {
-  int i = 0;
-  p.L = par[i++]; p.dt = par[i++];
-  for (int a = 0; a < 4; ++a) for (int b = 0; b < 4; ++b) p.pq[a][b] = par[i++];      // already symmetrised: Q + Q'
-  for (int a = 0; a < 2; ++a) for (int b = 0; b < 2; ++b) p.pr[a][b] = par[i++];
-  for (int a = 0; a < 4; ++a) for (int b = 0; b < 4; ++b) p.pqn[a][b] = par[i++];
-  for (int j = 0; j < 2; ++j) p.u_lo[j] = par[i++];
-  for (int j = 0; j < 2; ++j) p.u_hi[j] = par[i++];
-  p.v_lo = par[i++]; p.v_hi = par[i++];
-  for (int j = 0; j < 2; ++j) p.du_lo[j] = par[i++];
-  for (int j = 0; j < 2; ++j) p.du_hi[j] = par[i++];
-  p.w_v = par[i++]; p.w_u = par[i++]; p.w_du = par[i++];
-  p.N = N;
-  i = 0;
-  s.eps_abs = set[i++]; s.eps_rel = set[i++]; s.rho0 = set[i++]; s.alpha = set[i++]; s.sigma = set[i++];
-  s.adaptive_rho_tolerance = set[i++]; s.rho_eq_factor = set[i++]; s.rho_min = set[i++]; s.rho_max = set[i++];
-  s.delta = set[i++];
-  s.max_iter = (int)set[i++]; s.check_termination = (int)set[i++]; s.adaptive_rho = (int)set[i++];
-  s.adaptive_rho_interval = (int)set[i++]; s.polish_passes = (int)set[i++]; s.polish_refine_iter = (int)set[i++];
-  s.warm_start = (int)set[i++]; s.polish_retry = (int)set[i++]; s.early_polish = (int)set[i++]; s.early_polish_start = (int)set[i++];
-}
+static void unpack(const double* par, const double* set, int N, Params& p, Settings& s) { la::unpack(par, set, N, p, s); }
 
 static int g_fsave = 1;       // keep the ADMM factor in a side buffer over a polish (0: refactorise on resume)
 void emu_set_fsave(int f) { g_fsave = f; }
@@ -140,6 +117,69 @@ int emu_linearize_batch(const double* par, const double* set, int N, int B, cons
       a[2] = lin[0]; a[3] = lin[1]; a[6] = lin[2]; a[7] = lin[3];
       bm[2 * 2 + 1] = lin[4]; bm[3 * 2 + 0] = p.dt;
       cc[0] = lin[5]; cc[1] = lin[6]; cc[2] = 0.0; cc[3] = 0.0;
+    }
+  }
+  return 0;
+}
+
+// ---- linear solves one at a time (tests/test_linear_solves.py, la_systems.h), the sequential statements ------------------
+int emu_oe_doubles(int N) { return oe_doubles(N); }
+// bytes of mpc_exec.cuh GroupShared (a CUDA header): same members, same order
+int emu_group_shared_bytes() {
+  struct GS { int next; int anyv[2]; double red[2][8]; Drv drv; };
+  return (int)sizeof(GS);
+}
+
+// offsets (doubles from the workspace base) of the odd-even factor: dinv, sinv, gt, gb, and band_offset, oe_doubles
+int emu_oe_offsets(int N, int* o) {
+  std::vector<double> ws(footprint(N));
+  const View w = la::view(ws.data(), N);
+  const OEView oe = oe_view(w);
+  o[0] = (int)(oe.dinv - w.base); o[1] = (int)(oe.sinv - w.base); o[2] = (int)(oe.gt - w.base); o[3] = (int)(oe.gb - w.base);
+  o[4] = band_offset(N); o[5] = oe_doubles(N);
+  return 0;
+}
+
+// words of a problem's workspace (footprint(N)) that `mode` may change once its inputs are placed
+int emu_la_writable(int N, int mode, unsigned char* m) {
+  std::vector<double> ws(footprint(N));
+  la::writable(la::view(ws.data(), N), mode, m);
+  return 0;
+}
+
+// (A) reduced systems: S, F [nsys][J][36], b, x [nsys][J][6], fac [nsys][oe_doubles(N)] (the factor area afterwards)
+int emu_la_reduced(int N, int nsys, const double* S, const double* F, const double* b, double* x, double* fac) {
+  const int J = oe_neven(N), nf = oe_doubles(N);
+  std::vector<double> ws(footprint(N));
+  for (int i = 0; i < nsys; ++i) {
+    std::fill(ws.begin(), ws.end(), 0.0);
+    const View w = la::view(ws.data(), N);
+    for (int j = 0; j < J; ++j) la::red_place(w, S + (size_t)36 * J * i, F + (size_t)36 * J * i, b + (size_t)6 * J * i, j);
+    la::red_solve_seq(w);
+    for (int j = 0; j < J; ++j) la::red_read(w, x + (size_t)6 * J * i, j);
+    for (int t = 0; t < nf; ++t) fac[(size_t)nf * i + t] = (w.base + band_offset(N))[t];
+  }
+  return 0;
+}
+
+// (B) mode 1, ADMM operator at rho[i];  (C) mode 2, polish operator with activity words act [nsys][N+2].
+// x0 [nsys][4], ref [nsys][N+1][4], b, x [nsys][N+1][6]
+int emu_la_operator(int mode, const double* par, const double* set, int N, int nsys, const double* rho, const double* x0,
+                    const double* ref, const int* act, const double* b, double* x) {
+  Params p; Settings s; unpack(par, set, N, p, s);
+  std::vector<double> ws(footprint(N));
+  const size_t nb = (size_t)6 * (N + 1);
+  for (int i = 0; i < nsys; ++i) {
+    std::fill(ws.begin(), ws.end(), 0.0);
+    const View w = la::view(ws.data(), N);
+    la::prob_head(w, x0 + 4 * i, ref + (size_t)4 * (N + 1) * i, mode == la::MODE_POLISH ? act + (size_t)(N + 2) * i : nullptr);
+    for (int k = 0; k <= N; ++k) la::prob_stage(w, p, ref + (size_t)4 * (N + 1) * i, k);
+    if (mode == la::MODE_ADMM) {
+      la::admm_seq(w, p, s, rho[i], b + nb * i);
+      for (int k = 0; k <= N; ++k) la::admm_read(w, x + nb * i, k);
+    } else {
+      la::pol_seq(w, p, s, b + nb * i);
+      for (int k = 0; k <= N; ++k) la::pol_read(w, x + nb * i, k);
     }
   }
   return 0;
