@@ -9,6 +9,7 @@
  *                                (src/control/mpc_controller.py:39-141)
  *   cudampc_rollout_batch      <- TrajectoryTracker.track closed loop incl. _solve_with_relaxation
  *                                (src/pipeline/control_stage.py:33-56,74-157; vehicle_model.f_discrete :11-21)
+ *   cudampc_track_step_batch   <- one step of that loop with the plant left to the caller (control_stage.py:126-147)
  *   cudampc_build_reference_batch <- build_reference(path, desired_speed, horizon, dt) -> (M,4) rows [x,y,yaw,v_ref]
  *                                (src/control/ref_builder.py:10-22, src/common/geometry.py:9-45)
  *   cudampc_params            <- MPCParameters (src/control/mpc_controller.py:17-30; defaults src/config.py:66-92)
@@ -106,7 +107,7 @@ typedef struct cudampc_rollout_cfg {
   double relax_ddelta;      /* 0.05 */
   int32_t* step_ns_dev;     /* optional device array (B, sim_steps) int32: wall time of every closed-loop step of every vehicle
                                in nanoseconds (%globaltimer around window gather + solve (+ retry) + f_discrete + path-index
-                               rule), 0 for steps not run; NULL = not recorded.  What "p99 per-step latency" is measured from. */
+                               rule + goal test), 0 for steps not run; NULL = not recorded.  What "p99 per-step latency" is measured from. */
 } cudampc_rollout_cfg;
 
 typedef struct cudampc_handle cudampc_handle;
@@ -174,6 +175,32 @@ int cudampc_rollout_batch(cudampc_handle* h, int batch, const double* ref_global
                           const cudampc_settings* settings, const cudampc_rollout_cfg* cfg, double* states_dev,
                           double* controls_dev, int32_t* n_steps_dev, int32_t* flags_dev, int32_t* step_status_dev,
                           int32_t* step_iters_dev, void* stream);
+
+/* One closed-loop step of `batch` vehicles whose states come from a plant the caller owns (a simulator, a real vehicle, a
+ * model with mismatch or noise): the per-step half of cudampc_rollout_batch, one kernel launch per call.  Device pointers.
+ *   in : ref_global (B, ref_stride, 4) with ref_len[b] valid rows each, goal (B,2) as for cudampc_rollout_batch;
+ *        state (B,4) the measured state of every vehicle;
+ *        cfg: relax_on_failure, advance_dist2, goal_radius and relax_* are read (NULL = defaults); sim_steps and step_ns_dev
+ *        are not read.
+ *   in/out, the tracker state: path_idx (B) int32, u_prev (B,2), n_steps (B) int32, flags (B) int32 (the bits of
+ *        cudampc_rollout_batch).  The caller owns these arrays and zeroes them before the first step of a roll-out.
+ *   out: u0 (B,2); Xp (B,4,N+1) and Up (B,2,N) as cudampc_solve_batch, or NULL (not returned); status (B), iters (B) int32.
+ * Per vehicle: ref_len[b] < 1 sets flags = 2 (aborted) and solves nothing.  A stopped vehicle (flags bit 0 or 1) gets status 0,
+ * iters 0 and NaN u0 / Xp / Up, and its tracker state does not change.  From its second step on, the path-index rule and the
+ * goal test run on the measured state first (as cudampc_rollout_batch runs them after each step); a vehicle at the goal
+ * sets bit 0 and stops there.  Otherwise the window at path_idx is solved from the measured state and u_prev (+ the
+ * relaxation retry, bit 2).  On success u0 is carried into u_prev and n_steps grows by one; on failure bit 1 is set and
+ * u0 / Xp / Up are NaN (status and iters are those of the failed solve).  With f_discrete as the plant the steps reproduce
+ * cudampc_rollout_batch.
+ * Warm start (settings->warm_start = 1) uses the iterate the handle stored in slot b, the slot cudampc_solve_batch and
+ * cudampc_rollout_batch use for problem b: another call on the same handle between two steps changes the next step's
+ * starting point (and iteration count), not the optimum it converges to. */
+int cudampc_track_step_batch(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                             int ref_stride, const double* goal_dev, const double* state_dev,
+                             const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                             int32_t* path_idx_dev, double* u_prev_dev, int32_t* n_steps_dev, int32_t* flags_dev,
+                             double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                             void* stream);
 
 /* Introspection used by bench.py / tests: shared-memory doubles per problem, problems resident per SM,
  * number of kernel launches issued by this handle so far. */

@@ -36,7 +36,8 @@ class RolloutCfg(C.Structure):
 SYMBOLS = (
     "cudampc_version", "cudampc_default_settings", "cudampc_default_rollout_cfg", "cudampc_create",
     "cudampc_destroy", "cudampc_last_error", "cudampc_set_params", "cudampc_linearize_batch", "cudampc_f_discrete_batch",
-    "cudampc_solve_batch", "cudampc_solve_batch_host", "cudampc_build_reference_batch", "cudampc_rollout_batch", "cudampc_workspace_doubles",
+    "cudampc_solve_batch", "cudampc_solve_batch_host", "cudampc_build_reference_batch", "cudampc_rollout_batch",
+    "cudampc_track_step_batch", "cudampc_workspace_doubles",
     "cudampc_problems_per_sm", "cudampc_rollout_resident", "cudampc_launch_count", "cudampc_fp64_peak_tflops",
 )
 
@@ -80,6 +81,9 @@ def load() -> C.CDLL:
     lib.cudampc_rollout_batch.argtypes = [vp, C.c_int, dp, ip, C.c_int, dp, dp, C.POINTER(Settings),
                                           C.POINTER(RolloutCfg), dp, dp, ip, ip, ip, ip, vp]
     lib.cudampc_rollout_batch.restype = C.c_int
+    lib.cudampc_track_step_batch.argtypes = [vp, C.c_int, dp, ip, C.c_int, dp, dp, C.POINTER(Settings), C.POINTER(RolloutCfg),
+                                             ip, dp, ip, ip, dp, dp, dp, ip, ip, vp]
+    lib.cudampc_track_step_batch.restype = C.c_int
     lib.cudampc_workspace_doubles.argtypes = [vp]
     lib.cudampc_workspace_doubles.restype = C.c_int
     lib.cudampc_problems_per_sm.argtypes = [vp]

@@ -9,7 +9,9 @@ Mirror of /root/reference/src/pipeline/control_stage.py:26-157:
   failure :108-110);
 * new ``track_batch`` runs thousands of vehicles for all steps inside one CUDA launch
   (cudampc_rollout_batch): window gather + tail padding, solve with warm start, relaxation retry,
-  ``f_discrete``, ``u_prev`` carry, path-index rule and goal mask all stay on the device.
+  ``f_discrete``, ``u_prev`` carry, path-index rule and goal mask all stay on the device;
+* new ``start_batch`` returns a ``TrackingSession`` whose ``step(states)`` runs one closed-loop step of every vehicle from
+  states measured by a plant the caller owns (cudampc_track_step_batch), the tracker state staying on the device.
 """
 from __future__ import annotations
 
@@ -147,6 +149,29 @@ class TrajectoryTracker:
         return TrackingResult(states=states)
 
     # -- batched, device-resident closed loop ---------------------------------------------------------
+    def _references(self, ctl: MPCController, paths, ref_globals, build_on_device: bool):
+        """The global references of a batch on ``ctl``'s device: ``(ref (B, stride, 4), ref_len (B,), stride)``."""
+        import torch
+        N = ctl.params.horizon
+        if ref_globals is None and build_on_device:
+            # the reference's build_reference (ref_builder.py:10-22) for all paths in one launch (K_ref)
+            d_ref, d_len = ctl.build_reference_batch(paths, float(self.mpc.v_px_s))
+            return d_ref, d_len, int(d_ref.shape[1])
+        if ref_globals is None:
+            if any(len(p) < 1 for p in paths):
+                raise RuntimeError("Planner returned an empty path")   # control_stage.py:71-72
+            ref_globals = [build_reference(p, self.mpc.v_px_s, N, self.mpc.dt) for p in paths]
+        B = len(ref_globals)
+        if any(len(r) < 1 for r in ref_globals):
+            raise RuntimeError("Planner returned an empty path")
+        lens = np.array([len(r) for r in ref_globals], dtype=np.int32)
+        stride = int(lens.max())
+        refg = np.zeros((B, stride, 4))
+        for b, r in enumerate(ref_globals):
+            refg[b, :len(r)] = r
+        dev = torch.device("cuda", self.device)
+        return torch.as_tensor(refg).to(dev), torch.as_tensor(lens).to(dev), stride
+
     def track_batch(self, paths: Sequence, starts, goals, *, map_resolution: float, sim_steps: Optional[int] = None,
                     ref_globals: Optional[Sequence[np.ndarray]] = None, states0=None, warm_start: bool = True,
                     relax_on_failure: bool = True, build_on_device: bool = True, record_step_time: bool = False) -> BatchTrackingResult:
@@ -154,30 +179,12 @@ class TrajectoryTracker:
         ``(B,2)``.  Alternatively pass prebuilt ``ref_globals`` (each ``(M_b,4)``) and ``states0 (B,4)``."""
         import torch
         params = params_from_config(self.mpc, map_resolution)
-        N = params.horizon
         T = int(self.mpc.sim_steps if sim_steps is None else sim_steps)
         dev = torch.device("cuda", self.device)
         t = lambda a: torch.as_tensor(a).to(dev)
         ctl = self._controller(params, key="rollout")
-        if ref_globals is None and build_on_device:
-            # the reference's build_reference (ref_builder.py:10-22) for all paths in one launch (K_ref)
-            B = len(paths)
-            d_ref, d_len = ctl.build_reference_batch(paths, float(self.mpc.v_px_s))
-            stride = int(d_ref.shape[1])
-        else:
-            if ref_globals is None:
-                if any(len(p) < 1 for p in paths):
-                    raise RuntimeError("Planner returned an empty path")   # control_stage.py:71-72
-                ref_globals = [build_reference(p, self.mpc.v_px_s, N, self.mpc.dt) for p in paths]
-            B = len(ref_globals)
-            if any(len(r) < 1 for r in ref_globals):
-                raise RuntimeError("Planner returned an empty path")
-            lens = np.array([len(r) for r in ref_globals], dtype=np.int32)
-            stride = int(lens.max())
-            refg = np.zeros((B, stride, 4))
-            for b, r in enumerate(ref_globals):
-                refg[b, :len(r)] = r
-            d_ref, d_len = t(refg), t(lens)
+        d_ref, d_len, stride = self._references(ctl, paths, ref_globals, build_on_device)
+        B = int(d_ref.shape[0])
         if states0 is None:
             states0 = np.stack([initial_state(paths[b], starts[b]) for b in range(B)])
         states0 = np.ascontiguousarray(states0, dtype=np.float64).reshape(B, 4)
@@ -208,6 +215,117 @@ class TrajectoryTracker:
                                    step_status=d_st.cpu().numpy(), step_iters=d_it.cpu().numpy(), relaxed=(flags & 4).astype(bool),
                                    step_ns=d_ns.cpu().numpy() if d_ns is not None else None)
 
+    # -- one closed-loop step per call, the plant outside -----------------------------------------------
+    def start_batch(self, paths: Optional[Sequence], starts, goals, *, map_resolution: float,
+                    ref_globals: Optional[Sequence[np.ndarray]] = None, states0=None, warm_start: bool = True,
+                    relax_on_failure: bool = True, build_on_device: bool = True) -> "TrackingSession":
+        """Start tracking ``B`` vehicles whose states come from a plant the caller owns (a simulator, a real vehicle, a model
+        with mismatch or noise).  References, starts and goals as ``track_batch``; ``session.step(states)`` then runs one
+        closed-loop step of every vehicle in one launch (cudampc_track_step_batch).  ``session.states0`` is the initial state
+        of every vehicle (``initial_state`` of its path unless ``states0`` is given), the plant's first input."""
+        import torch
+        params = params_from_config(self.mpc, map_resolution)
+        # the session's own handle: nobody else reuses the warm-start slots of its vehicles between steps
+        B = len(ref_globals) if ref_globals is not None else len(paths)
+        ctl = MPCController(params, self.settings, device=self.device, max_batch=max(B, 1))
+        d_ref, d_len, stride = self._references(ctl, paths, ref_globals, build_on_device)
+        if states0 is None:
+            states0 = np.stack([initial_state(paths[b], starts[b]) for b in range(B)]) if B else np.zeros((0, 4))
+        states0 = np.ascontiguousarray(states0, dtype=np.float64).reshape(B, 4)
+        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(B, 2)
+        s = replace(self.settings or SolverSettings(), warm_start=warm_start).to_c()
+        cfg = _lib.RolloutCfg()
+        _lib.load().cudampc_default_rollout_cfg(C.byref(cfg))
+        cfg.relax_on_failure = int(relax_on_failure)
+        return TrackingSession(ctl, d_ref, d_len, stride, torch.as_tensor(goals).to(d_ref.device), states0, s, cfg)
+
+
+@dataclass
+class StepResult:
+    """What one ``TrackingSession.step`` returns (CUDA tensors for CUDA input, NumPy arrays for NumPy input).  A vehicle that
+    did not step (stopped before, at the goal now, or the solve failed) has NaN ``u0``, ``Xp`` and ``Up``; ``status`` is 0
+    when no solve ran."""
+    u0: object       # (B,2)
+    Xp: object       # (B,4,N+1) state-major predicted trajectory
+    Up: object       # (B,2,N)
+    status: object   # (B,) int32 OSQP codes
+    iters: object    # (B,) int32
+
+
+class TrackingSession:
+    """The tracker state of ``B`` vehicles on the device between the steps of an external plant (``TrajectoryTracker.start_batch``).
+
+    ``path_idx``, ``u_prev``, ``n_steps`` and the flag views are CUDA tensors; reading them does not synchronise."""
+
+    def __init__(self, ctl: MPCController, ref, ref_len, stride: int, goals, states0: np.ndarray, settings: _lib.Settings,
+                 cfg: _lib.RolloutCfg):
+        import torch
+        self.controller, self._ref, self._ref_len, self._stride, self._goals = ctl, ref, ref_len, int(stride), goals
+        self._settings, self._cfg = settings, cfg
+        self.states0 = states0
+        self.batch = B = int(ref.shape[0])
+        self.horizon = N = ctl.params.horizon
+        dev = self.device = ref.device
+        self.path_idx = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.u_prev = torch.zeros((B, 2), dtype=torch.float64, device=dev)
+        self.n_steps = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.flags = torch.zeros(B, dtype=torch.int32, device=dev)   # bit0 goal reached, bit1 aborted, bit2 relaxation ran
+        self._h = ctl._handle(max(B, 1))
+
+    @property
+    def goal_reached(self):
+        return (self.flags & 1) != 0
+
+    @property
+    def aborted(self):
+        return (self.flags & 2) != 0
+
+    @property
+    def relaxed(self):
+        return (self.flags & 4) != 0
+
+    @property
+    def active(self):
+        return (self.flags & 3) == 0
+
+    def launch_count(self) -> int:
+        return self.controller.launch_count()
+
+    def step(self, states) -> StepResult:
+        """One closed-loop step of every vehicle from its measured ``states (B,4)``.  A contiguous CUDA float64 tensor on the
+        session's device: asynchronous on the current stream, CUDA tensors out.  A NumPy float64 array: copied in, synchronised,
+        NumPy out."""
+        import torch
+        B, N = self.batch, self.horizon
+        host = isinstance(states, np.ndarray)
+        if host:
+            if states.shape != (B, 4) or states.dtype != np.float64:
+                raise ValueError(f"states: expected a float64 array of shape ({B}, 4); got {states.dtype} {states.shape}")
+            x = torch.as_tensor(np.ascontiguousarray(states)).to(self.device)
+        elif isinstance(states, torch.Tensor):
+            if tuple(states.shape) != (B, 4) or states.dtype != torch.float64 or states.device != self.device or not states.is_contiguous():
+                raise ValueError(f"states: expected a contiguous float64 tensor of shape ({B}, 4) on {self.device}; "
+                                 f"got {states.dtype} {tuple(states.shape)} on {states.device}")
+            x = states
+        else:
+            raise ValueError(f"states: expected a NumPy array or a CUDA tensor; got {type(states).__name__}")
+        e = lambda *shape, dt=torch.float64: torch.empty(shape, dtype=dt, device=self.device)
+        out = StepResult(e(B, 2), e(B, 4, N + 1), e(B, 2, N), e(B, dt=torch.int32), e(B, dt=torch.int32))
+        if B:
+            h = self._h
+            p = lambda t: C.c_void_p(t.data_ptr())
+            rc = h.lib.cudampc_track_step_batch(h.ptr, B, p(self._ref), p(self._ref_len), self._stride, p(self._goals), p(x),
+                                                C.byref(self._settings), C.byref(self._cfg), p(self.path_idx), p(self.u_prev),
+                                                p(self.n_steps), p(self.flags), p(out.u0), p(out.Xp), p(out.Up), p(out.status),
+                                                p(out.iters), C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
+            _lib.check(h.lib, h.ptr, rc, "cudampc_track_step_batch")
+        if host:
+            return StepResult(*(t.cpu().numpy() for t in (out.u0, out.Xp, out.Up, out.status, out.iters)))
+        return out
+
+    def close(self) -> None:
+        self.controller.close()
+
 
 def _reference_plotter():
     """The reference's own plotting (src/viz, untouched) when this module is dropped into the reference tree."""
@@ -224,4 +342,4 @@ def _reference_plotter():
     return plot
 
 
-__all__ = ["TrajectoryTracker", "TrackingResult", "BatchTrackingResult", "initial_state"]
+__all__ = ["TrajectoryTracker", "TrackingResult", "BatchTrackingResult", "TrackingSession", "StepResult", "initial_state"]

@@ -194,6 +194,10 @@ cudaError_t rollout_occupancy_short(int, int*), rollout_occupancy_general(int, i
 void rollout_launch_short(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
 void rollout_launch_general(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
 void rollout_launch_pair(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
+cudaError_t step_set_smem_short(int), step_set_smem_general(int), step_set_smem_pair(int);
+void step_launch_short(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
+void step_launch_general(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
+void step_launch_pair(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
 cudaError_t solve_set_smem(int v, int bytes) { return v == 0 ? solve_set_smem_0(bytes) : v == 1 ? solve_set_smem_1(bytes) : v == 2 ? solve_set_smem_2(bytes) : v == 3 ? solve_set_smem_3(bytes) : v == 4 ? solve_set_smem_4(bytes) : solve_set_smem_5(bytes); }
 void solve_launch(int v, int grid, int threads, int smem, cudaStream_t st, const Params& p, const Settings& s, const BatchArgs& a, int P, int F) {
   if (v == 0) solve_launch_0(grid, threads, smem, st, p, s, a, P, F);
@@ -211,6 +215,12 @@ void rollout_launch(int f, int grid, int smem, cudaStream_t st, const Params& p,
   if (f == FORM_SHORT) rollout_launch_short(grid, smem, st, p, s, cfg, a);
   else if (f == FORM_PAIR) rollout_launch_pair(grid, smem, st, p, s, cfg, a);
   else rollout_launch_general(grid, smem, st, p, s, cfg, a);
+}
+cudaError_t step_set_smem(int f, int bytes) { return f == FORM_SHORT ? step_set_smem_short(bytes) : f == FORM_PAIR ? step_set_smem_pair(bytes) : step_set_smem_general(bytes); }
+void step_launch(int f, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a) {
+  if (f == FORM_SHORT) step_launch_short(grid, smem, st, p, s, cfg, a);
+  else if (f == FORM_PAIR) step_launch_pair(grid, smem, st, p, s, cfg, a);
+  else step_launch_general(grid, smem, st, p, s, cfg, a);
 }
 
 // Every entry point runs on the handle's device and leaves the caller's current device as it found it.
@@ -370,6 +380,7 @@ int cudampc_create(const cudampc_params* params, int max_batch, int device, cuda
     else if (!strcmp(fe, "short") && p.N + 1 <= 32) h->form = FORM_SHORT;
   }
   e = rollout_set_smem(h->form, h->smem_bytes);
+  if (e == cudaSuccess) e = step_set_smem(h->form, h->smem_bytes);     // K_step: K_rollout's form and workspace
   int occ = 0;
   if (e == cudaSuccess) e = rollout_occupancy(h->form, h->smem_bytes, &occ);
   if (e != cudaSuccess || occ < 1) { delete h; return fail(nullptr, CUDAMPC_ERR_CUDA, "CUDA failure: %s", cudaGetErrorString(e)); }
@@ -656,6 +667,39 @@ int cudampc_rollout_batch(cudampc_handle* h, int batch, const double* ref_global
     if (grid > batch) grid = batch;
     rollout_launch(h->form, grid, h->smem_bytes, st, h->p, s, c, a);
   }
+  h->launches++;
+  CU(h, cudaGetLastError());
+  return CUDAMPC_OK;
+}
+
+int cudampc_track_step_batch(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                             int ref_stride, const double* goal_dev, const double* state_dev,
+                             const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                             int32_t* path_idx_dev, double* u_prev_dev, int32_t* n_steps_dev, int32_t* flags_dev,
+                             double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                             void* stream) {
+  if (!h) return CUDAMPC_ERR_INVALID;
+  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s", "track_step_batch: batch out of range for this handle");
+  if (!ref_global_dev || !ref_len_dev || !goal_dev || !state_dev || !path_idx_dev || !u_prev_dev || !n_steps_dev || !flags_dev ||
+      !u0_dev || !status_dev || !iters_dev || ref_stride < 1)
+    return fail(h, CUDAMPC_ERR_INVALID, "%s", "track_step_batch: NULL pointer or bad stride");
+  cudampc_rollout_cfg c;
+  if (cfg) c = *cfg; else cudampc_default_rollout_cfg(&c);
+  Settings s;
+  int rc = convert_settings(settings, &s, h);
+  if (rc) return rc;
+  if (batch == 0) return CUDAMPC_OK;
+  ON_DEVICE(h);
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(h, cudaMemsetAsync(h->counter, 0, sizeof(int), st));
+  StepArgs a;
+  a.ref_global = ref_global_dev; a.ref_len = ref_len_dev; a.ref_stride = ref_stride; a.goal = goal_dev; a.state = state_dev;
+  a.warm = h->warm; a.scratch = h->scratch; a.fsave = getenv("CUDAMPC_NO_FSAVE") ? nullptr : h->fsave; a.work = h->work;
+  a.path_idx = path_idx_dev; a.u_prev = u_prev_dev; a.n_steps = n_steps_dev; a.flags = flags_dev;
+  a.u0 = u0_dev; a.Xp = Xp_dev; a.Up = Up_dev; a.status = status_dev; a.iters = iters_dev; a.counter = h->counter; a.batch = batch;
+  int grid = h->sms * h->roll_per_sm;
+  if (grid > batch) grid = batch;
+  step_launch(h->form, grid, h->smem_bytes, st, h->p, s, c, a);
   h->launches++;
   CU(h, cudaGetLastError());
   return CUDAMPC_OK;

@@ -1,4 +1,4 @@
-// mpc_kernels_tu.cu — one instantiation of K_solve / K_rollout per translation unit (nvcc -DMPC_TU=n; see mpc_kernels.cuh).
+// mpc_kernels_tu.cu — one instantiation of K_solve / K_rollout (+ K_step) per translation unit (nvcc -DMPC_TU=n; see mpc_kernels.cuh).
 #include "mpc_kernels.cuh"
 #ifndef MPC_REG_MAXT
 #define MPC_REG_MAXT 256       // register form: threads per CTA the kernel is compiled for (256: 255 registers, 4 problems; 320 / 384: 168 registers)
@@ -23,6 +23,10 @@
   cudaError_t rollout_occupancy_##name(int bytes, int* n) { return cudaOccupancyMaxActiveBlocksPerMultiprocessor(n, mpc_rollout_kernel<FORM>, 32, bytes); } \
   void rollout_launch_##name(int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const RolloutArgs& a) { \
     mpc_rollout_kernel<FORM><<<grid, 32, smem, st>>>(p, s, cfg, a);                                                          \
+  }                                                                                                                          \
+  cudaError_t step_set_smem_##name(int bytes) { return cudaFuncSetAttribute(mpc_track_step_kernel<FORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); } \
+  void step_launch_##name(int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a) { \
+    mpc_track_step_kernel<FORM><<<grid, 32, smem, st>>>(p, s, cfg, a);                                                       \
   }
 
 #if MPC_TU == 0
