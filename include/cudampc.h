@@ -46,7 +46,9 @@ enum {
   CUDAMPC_SOLVED = 1,
   CUDAMPC_SOLVED_INACCURATE = 2,
   CUDAMPC_MAX_ITER_REACHED = -2,
-  CUDAMPC_UNSOLVED = -10
+  CUDAMPC_UNSOLVED = -10,
+  CUDAMPC_INVALID_PARAMS = -100 /* not an OSQP code: the problem's own parameter record was rejected (the *_params entry
+                                   points), nothing was solved */
 };
 
 /* Mirror of MPCParameters, field for field (mpc_controller.py:17-30). Matrices row-major. */
@@ -122,7 +124,8 @@ int cudampc_create(const cudampc_params* params, int max_batch, int device, cuda
 int cudampc_destroy(cudampc_handle* h);
 const char* cudampc_last_error(const cudampc_handle* h); /* h may be NULL: message of the last failed create */
 
-/* Replace the parameters (same horizon) — used by the relaxation fallback and by callers that sweep limits. */
+/* Replace the parameters (same horizon) — used by the relaxation fallback and by callers that sweep limits (the *_params calls
+ * below run a sweep, or a fleet whose vehicles differ, in one launch). */
 int cudampc_set_params(cudampc_handle* h, const cudampc_params* params);
 
 /* (A_k, B_k, c_k), k = 0..N-1, exactly as MPCController.solve linearises them: stage k at the unwrapped
@@ -168,7 +171,9 @@ int cudampc_build_reference_batch(cudampc_handle* h, int batch, const double* pa
  *        state0 (B,4); goal (B,2)
  *   out: states (B, sim_steps, 4) post-step states (rows after a vehicle stops are NaN);
  *        controls (B, sim_steps, 2) or NULL; n_steps (B) int32 = len(TrackingResult.states);
- *        flags (B) int32: bit0 goal reached, bit1 aborted on solver failure, bit2 the relaxation retry ran at least once;
+ *        flags (B) int32: bit0 goal reached, bit1 aborted on solver failure, bit2 the relaxation retry ran at least once,
+ *        bit3 the vehicle's parameter record was rejected (cudampc_rollout_batch_params / _track_step_batch_params; set with
+ *        bit1, the vehicle takes no step);
  *        step_status (B, sim_steps) int32 or NULL; step_iters (B, sim_steps) int32 or NULL. */
 int cudampc_rollout_batch(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
                           int ref_stride, const double* state0_dev, const double* goal_dev,
@@ -201,6 +206,34 @@ int cudampc_track_step_batch(cudampc_handle* h, int batch, const double* ref_glo
                              int32_t* path_idx_dev, double* u_prev_dev, int32_t* n_steps_dev, int32_t* flags_dev,
                              double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
                              void* stream);
+
+/* Per-problem parameters: the same calls as cudampc_solve_batch, cudampc_rollout_batch and cudampc_track_step_batch, where
+ * problem (or vehicle) b is solved with its own record params_dev[b] instead of the handle's parameters.
+ *   params_dev: device array of `batch` cudampc_params records, in problem order for the solve and in vehicle order for the
+ *   roll-out and the step.  Every field may differ from the handle's except horizon and dt: the horizon fixes the workspace
+ *   layout, dt the time grid of the references and of a step.  A record is accepted by the rules cudampc_create applies
+ *   (dt, wheelbase_px > 0; q, q_terminal, r positive semidefinite and non-zero; slack weights > 0) and only if its horizon
+ *   equals the handle's and its dt compares equal to the handle's.
+ * A rejected record fails only its own problem, inside the launch: the solve returns status CUDAMPC_INVALID_PARAMS, iters 0,
+ * NaN u0 / Xp / Up / pri_res / dua_res and zero info, and leaves the problem's warm-start slot unchanged; a vehicle of the
+ * roll-out or the step takes no step and gets flags bits 1 and 3 and the outputs of a vehicle with an empty path.
+ * One launch per call, as the shared-parameter calls; the records are read and checked inside it. */
+int cudampc_solve_batch_params(cudampc_handle* h, int batch, const double* x0_dev, const double* ref_dev,
+                               const double* u_prev_dev, const cudampc_settings* settings, const cudampc_params* params_dev,
+                               double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                               double* pri_res_dev, double* dua_res_dev, int32_t* info_dev, void* stream);
+int cudampc_rollout_batch_params(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                                 int ref_stride, const double* state0_dev, const double* goal_dev,
+                                 const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                                 const cudampc_params* params_dev, double* states_dev, double* controls_dev,
+                                 int32_t* n_steps_dev, int32_t* flags_dev, int32_t* step_status_dev, int32_t* step_iters_dev,
+                                 void* stream);
+int cudampc_track_step_batch_params(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                                    int ref_stride, const double* goal_dev, const double* state_dev,
+                                    const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                                    const cudampc_params* params_dev, int32_t* path_idx_dev, double* u_prev_dev,
+                                    int32_t* n_steps_dev, int32_t* flags_dev, double* u0_dev, double* Xp_dev, double* Up_dev,
+                                    int32_t* status_dev, int32_t* iters_dev, void* stream);
 
 /* Introspection used by bench.py / tests: shared-memory doubles per problem, problems resident per SM,
  * number of kernel launches issued by this handle so far. */

@@ -5,6 +5,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CUDAMPC_LIB") or os.path.join(_HERE, "libcudampc.so")      # CUDAMPC_LIB: dev builds (timing, poison)
 
@@ -14,6 +16,15 @@ class Params(C.Structure):
                 ("q", C.c_double * 16), ("r", C.c_double * 4), ("q_terminal", C.c_double * 16),
                 ("u_bounds", C.c_double * 4), ("v_bounds", C.c_double * 2), ("du_bounds", C.c_double * 4),
                 ("slack_velocity", C.c_double), ("slack_input", C.c_double), ("slack_rate", C.c_double)]
+
+
+# the same record as a NumPy structured dtype (arrays of per-problem parameters, field-wise editable: arr["du_bounds"][:, 3] = ...)
+PARAMS_DTYPE = np.dtype([(name, np.float64 if t is C.c_double else np.int32 if t is C.c_int32 else (np.float64, (t._length_,)))
+                         for name, t in Params._fields_], align=True)
+assert PARAMS_DTYPE.itemsize == C.sizeof(Params)
+
+# status of a problem whose own parameter record was rejected (CUDAMPC_INVALID_PARAMS)
+STATUS_INVALID_PARAMS = -100
 
 
 class Settings(C.Structure):
@@ -37,7 +48,8 @@ SYMBOLS = (
     "cudampc_version", "cudampc_default_settings", "cudampc_default_rollout_cfg", "cudampc_create",
     "cudampc_destroy", "cudampc_last_error", "cudampc_set_params", "cudampc_linearize_batch", "cudampc_f_discrete_batch",
     "cudampc_solve_batch", "cudampc_solve_batch_host", "cudampc_build_reference_batch", "cudampc_rollout_batch",
-    "cudampc_track_step_batch", "cudampc_workspace_doubles",
+    "cudampc_track_step_batch", "cudampc_solve_batch_params", "cudampc_rollout_batch_params", "cudampc_track_step_batch_params",
+    "cudampc_workspace_doubles",
     "cudampc_problems_per_sm", "cudampc_rollout_resident", "cudampc_launch_count", "cudampc_fp64_peak_tflops",
 )
 
@@ -84,6 +96,14 @@ def load() -> C.CDLL:
     lib.cudampc_track_step_batch.argtypes = [vp, C.c_int, dp, ip, C.c_int, dp, dp, C.POINTER(Settings), C.POINTER(RolloutCfg),
                                              ip, dp, ip, ip, dp, dp, dp, ip, ip, vp]
     lib.cudampc_track_step_batch.restype = C.c_int
+    lib.cudampc_solve_batch_params.argtypes = [vp, C.c_int, dp, dp, dp, C.POINTER(Settings), vp, dp, dp, dp, ip, ip, dp, dp, ip, vp]
+    lib.cudampc_solve_batch_params.restype = C.c_int
+    lib.cudampc_rollout_batch_params.argtypes = [vp, C.c_int, dp, ip, C.c_int, dp, dp, C.POINTER(Settings),
+                                                 C.POINTER(RolloutCfg), vp, dp, dp, ip, ip, ip, ip, vp]
+    lib.cudampc_rollout_batch_params.restype = C.c_int
+    lib.cudampc_track_step_batch_params.argtypes = [vp, C.c_int, dp, ip, C.c_int, dp, dp, C.POINTER(Settings), C.POINTER(RolloutCfg),
+                                                    vp, ip, dp, ip, ip, dp, dp, dp, ip, ip, vp]
+    lib.cudampc_track_step_batch_params.restype = C.c_int
     lib.cudampc_workspace_doubles.argtypes = [vp]
     lib.cudampc_workspace_doubles.restype = C.c_int
     lib.cudampc_problems_per_sm.argtypes = [vp]

@@ -24,7 +24,7 @@ import numpy as np
 
 from . import _lib
 from .config import params_from_config
-from .mpc_controller import MPCController, MPCParameters, SolverSettings, params_to_c
+from .mpc_controller import MPCController, MPCParameters, SolverSettings, params_rows, params_to_c, params_to_device
 from .ref_builder import build_reference
 from .vehicle_model import f_discrete
 
@@ -49,6 +49,7 @@ class BatchTrackingResult:
     step_iters: np.ndarray    # (B, T) int32
     relaxed: Optional[np.ndarray] = None   # (B,) bool: the relaxation retry (control_stage.py:45-56) ran at least once
     step_ns: Optional[np.ndarray] = None   # (B, T) int32: wall time of every closed-loop step on the device (ns), if recorded
+    invalid_params: Optional[np.ndarray] = None   # (B,) bool: the vehicle's own parameters were rejected; it took no step (aborted)
 
     def result(self, b: int) -> TrackingResult:
         return TrackingResult(states=[self.states[b, t].copy() for t in range(int(self.n_steps[b]))])
@@ -174,17 +175,23 @@ class TrajectoryTracker:
 
     def track_batch(self, paths: Sequence, starts, goals, *, map_resolution: float, sim_steps: Optional[int] = None,
                     ref_globals: Optional[Sequence[np.ndarray]] = None, states0=None, warm_start: bool = True,
-                    relax_on_failure: bool = True, build_on_device: bool = True, record_step_time: bool = False) -> BatchTrackingResult:
+                    relax_on_failure: bool = True, build_on_device: bool = True, record_step_time: bool = False,
+                    vehicle_params=None) -> BatchTrackingResult:
         """Track ``B`` vehicles. ``paths[b]`` is a polyline (as ``PlanResult.path``); ``starts``/``goals`` are
-        ``(B,2)``.  Alternatively pass prebuilt ``ref_globals`` (each ``(M_b,4)``) and ``states0 (B,4)``."""
+        ``(B,2)``.  Alternatively pass prebuilt ``ref_globals`` (each ``(M_b,4)``) and ``states0 (B,4)``.
+
+        ``vehicle_params``: vehicle b's own ``MPCParameters`` (wheelbase, limits, weights; the relaxation retry widens its own
+        ``du_bounds``), as ``MPCController.solve_batch(params=...)`` takes them; horizon and dt must be those of ``self.mpc``.
+        A vehicle whose parameters the rules reject takes no step and is reported in ``invalid_params`` (and ``aborted``)."""
         import torch
         params = params_from_config(self.mpc, map_resolution)
         T = int(self.mpc.sim_steps if sim_steps is None else sim_steps)
         dev = torch.device("cuda", self.device)
         t = lambda a: torch.as_tensor(a).to(dev)
         ctl = self._controller(params, key="rollout")
+        B = len(ref_globals) if ref_globals is not None else len(paths)
+        rows = None if vehicle_params is None else params_rows(vehicle_params, B, params)
         d_ref, d_len, stride = self._references(ctl, paths, ref_globals, build_on_device)
-        B = int(d_ref.shape[0])
         if states0 is None:
             states0 = np.stack([initial_state(paths[b], starts[b]) for b in range(B)])
         states0 = np.ascontiguousarray(states0, dtype=np.float64).reshape(B, 4)
@@ -204,29 +211,40 @@ class TrajectoryTracker:
         d_ns = torch.zeros((B, T), dtype=torch.int32, device=dev) if record_step_time else None
         cfg.step_ns_dev = d_ns.data_ptr() if d_ns is not None else None
         p = lambda x: C.c_void_p(x.data_ptr())
-        rc = h.lib.cudampc_rollout_batch(h.ptr, B, p(d_ref), p(d_len), stride, p(d_s0), p(d_goal), C.byref(s), C.byref(cfg),
-                                         p(d_states), p(d_ctrl), p(d_n), p(d_fl), p(d_st), p(d_it),
-                                         C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
-        _lib.check(h.lib, h.ptr, rc, "cudampc_rollout_batch")
+        if rows is None:
+            rc = h.lib.cudampc_rollout_batch(h.ptr, B, p(d_ref), p(d_len), stride, p(d_s0), p(d_goal), C.byref(s), C.byref(cfg),
+                                             p(d_states), p(d_ctrl), p(d_n), p(d_fl), p(d_st), p(d_it),
+                                             C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _lib.check(h.lib, h.ptr, rc, "cudampc_rollout_batch")
+        else:
+            d_par = params_to_device(rows, dev)
+            rc = h.lib.cudampc_rollout_batch_params(h.ptr, B, p(d_ref), p(d_len), stride, p(d_s0), p(d_goal), C.byref(s), C.byref(cfg),
+                                                    p(d_par), p(d_states), p(d_ctrl), p(d_n), p(d_fl), p(d_st), p(d_it),
+                                                    C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _lib.check(h.lib, h.ptr, rc, "cudampc_rollout_batch_params")
         torch.cuda.synchronize(dev)
         flags = d_fl.cpu().numpy()
         return BatchTrackingResult(states=d_states.cpu().numpy(), controls=d_ctrl.cpu().numpy(), n_steps=d_n.cpu().numpy(),
                                    goal_reached=(flags & 1).astype(bool), aborted=(flags & 2).astype(bool),
                                    step_status=d_st.cpu().numpy(), step_iters=d_it.cpu().numpy(), relaxed=(flags & 4).astype(bool),
-                                   step_ns=d_ns.cpu().numpy() if d_ns is not None else None)
+                                   step_ns=d_ns.cpu().numpy() if d_ns is not None else None, invalid_params=(flags & 8).astype(bool))
 
     # -- one closed-loop step per call, the plant outside -----------------------------------------------
     def start_batch(self, paths: Optional[Sequence], starts, goals, *, map_resolution: float,
                     ref_globals: Optional[Sequence[np.ndarray]] = None, states0=None, warm_start: bool = True,
-                    relax_on_failure: bool = True, build_on_device: bool = True) -> "TrackingSession":
+                    relax_on_failure: bool = True, build_on_device: bool = True, vehicle_params=None) -> "TrackingSession":
         """Start tracking ``B`` vehicles whose states come from a plant the caller owns (a simulator, a real vehicle, a model
         with mismatch or noise).  References, starts and goals as ``track_batch``; ``session.step(states)`` then runs one
         closed-loop step of every vehicle in one launch (cudampc_track_step_batch).  ``session.states0`` is the initial state
-        of every vehicle (``initial_state`` of its path unless ``states0`` is given), the plant's first input."""
+        of every vehicle (``initial_state`` of its path unless ``states0`` is given), the plant's first input.
+        ``vehicle_params``: per-vehicle parameters as ``track_batch`` takes them; the session uploads them once and every
+        ``step`` solves each vehicle with its own (cudampc_track_step_batch_params).  A plant that integrates with
+        ``f_discrete`` then uses each vehicle's own wheelbase."""
         import torch
         params = params_from_config(self.mpc, map_resolution)
         # the session's own handle: nobody else reuses the warm-start slots of its vehicles between steps
         B = len(ref_globals) if ref_globals is not None else len(paths)
+        rows = None if vehicle_params is None else params_rows(vehicle_params, B, params)
         ctl = MPCController(params, self.settings, device=self.device, max_batch=max(B, 1))
         d_ref, d_len, stride = self._references(ctl, paths, ref_globals, build_on_device)
         if states0 is None:
@@ -237,7 +255,8 @@ class TrajectoryTracker:
         cfg = _lib.RolloutCfg()
         _lib.load().cudampc_default_rollout_cfg(C.byref(cfg))
         cfg.relax_on_failure = int(relax_on_failure)
-        return TrackingSession(ctl, d_ref, d_len, stride, torch.as_tensor(goals).to(d_ref.device), states0, s, cfg)
+        d_par = None if rows is None else params_to_device(rows, d_ref.device)
+        return TrackingSession(ctl, d_ref, d_len, stride, torch.as_tensor(goals).to(d_ref.device), states0, s, cfg, d_par)
 
 
 @dataclass
@@ -258,9 +277,10 @@ class TrackingSession:
     ``path_idx``, ``u_prev``, ``n_steps`` and the flag views are CUDA tensors; reading them does not synchronise."""
 
     def __init__(self, ctl: MPCController, ref, ref_len, stride: int, goals, states0: np.ndarray, settings: _lib.Settings,
-                 cfg: _lib.RolloutCfg):
+                 cfg: _lib.RolloutCfg, params=None):
         import torch
         self.controller, self._ref, self._ref_len, self._stride, self._goals = ctl, ref, ref_len, int(stride), goals
+        self._params = params     # per-vehicle records on the device (uint8 (B, 416)) or None
         self._settings, self._cfg = settings, cfg
         self.states0 = states0
         self.batch = B = int(ref.shape[0])
@@ -269,7 +289,7 @@ class TrackingSession:
         self.path_idx = torch.zeros(B, dtype=torch.int32, device=dev)
         self.u_prev = torch.zeros((B, 2), dtype=torch.float64, device=dev)
         self.n_steps = torch.zeros(B, dtype=torch.int32, device=dev)
-        self.flags = torch.zeros(B, dtype=torch.int32, device=dev)   # bit0 goal reached, bit1 aborted, bit2 relaxation ran
+        self.flags = torch.zeros(B, dtype=torch.int32, device=dev)   # bit0 goal reached, bit1 aborted, bit2 relaxation ran, bit3 invalid parameters
         self._h = ctl._handle(max(B, 1))
 
     @property
@@ -283,6 +303,10 @@ class TrackingSession:
     @property
     def relaxed(self):
         return (self.flags & 4) != 0
+
+    @property
+    def invalid_params(self):
+        return (self.flags & 8) != 0
 
     @property
     def active(self):
@@ -314,11 +338,19 @@ class TrackingSession:
         if B:
             h = self._h
             p = lambda t: C.c_void_p(t.data_ptr())
-            rc = h.lib.cudampc_track_step_batch(h.ptr, B, p(self._ref), p(self._ref_len), self._stride, p(self._goals), p(x),
-                                                C.byref(self._settings), C.byref(self._cfg), p(self.path_idx), p(self.u_prev),
-                                                p(self.n_steps), p(self.flags), p(out.u0), p(out.Xp), p(out.Up), p(out.status),
-                                                p(out.iters), C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
-            _lib.check(h.lib, h.ptr, rc, "cudampc_track_step_batch")
+            st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+            if self._params is None:
+                rc = h.lib.cudampc_track_step_batch(h.ptr, B, p(self._ref), p(self._ref_len), self._stride, p(self._goals), p(x),
+                                                    C.byref(self._settings), C.byref(self._cfg), p(self.path_idx), p(self.u_prev),
+                                                    p(self.n_steps), p(self.flags), p(out.u0), p(out.Xp), p(out.Up), p(out.status),
+                                                    p(out.iters), st)
+                _lib.check(h.lib, h.ptr, rc, "cudampc_track_step_batch")
+            else:
+                rc = h.lib.cudampc_track_step_batch_params(h.ptr, B, p(self._ref), p(self._ref_len), self._stride, p(self._goals), p(x),
+                                                           C.byref(self._settings), C.byref(self._cfg), p(self._params),
+                                                           p(self.path_idx), p(self.u_prev), p(self.n_steps), p(self.flags), p(out.u0),
+                                                           p(out.Xp), p(out.Up), p(out.status), p(out.iters), st)
+                _lib.check(h.lib, h.ptr, rc, "cudampc_track_step_batch_params")
         if host:
             return StepResult(*(t.cpu().numpy() for t in (out.u0, out.Xp, out.Up, out.status, out.iters)))
         return out

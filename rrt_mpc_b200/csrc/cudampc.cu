@@ -172,6 +172,10 @@ struct cudampc_handle {
   int sms, smem_bytes, roll_per_sm;   // K_rollout: one-warp CTAs of smem_bytes each, roll_per_sm resident per SM
   int grp_P, grp_wpp, grp_smem;        // K_solve: one CTA per SM with grp_P groups of grp_wpp warps
   int variant;                         // SolveVariant
+  // per-problem-parameter kernels (the *_params entry points), configured on first use: a Params slot per group / CTA on top of
+  // the shared-parameter layout, so at most as many groups and resident CTAs as above (the allocations are sized for those)
+  bool pp_ready;
+  int pp_P, pp_smem, pp_roll_per_sm, pp_roll_smem;
   int form;                            // form of the ADMM phases (mpc_solve.h FORM_*): K_solve one-warp groups, K_rollout
   unsigned long long* tags;            // dev builds (MPC_TIMING): per-tag cycle counters
   long long launches;
@@ -198,27 +202,62 @@ cudaError_t step_set_smem_short(int), step_set_smem_general(int), step_set_smem_
 void step_launch_short(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
 void step_launch_general(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
 void step_launch_pair(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
-cudaError_t solve_set_smem(int v, int bytes) { return v == 0 ? solve_set_smem_0(bytes) : v == 1 ? solve_set_smem_1(bytes) : v == 2 ? solve_set_smem_2(bytes) : v == 3 ? solve_set_smem_3(bytes) : v == 4 ? solve_set_smem_4(bytes) : solve_set_smem_5(bytes); }
-void solve_launch(int v, int grid, int threads, int smem, cudaStream_t st, const Params& p, const Settings& s, const BatchArgs& a, int P, int F) {
-  if (v == 0) solve_launch_0(grid, threads, smem, st, p, s, a, P, F);
-  else if (v == 1) solve_launch_1(grid, threads, smem, st, p, s, a, P, F);
-  else if (v == 2) solve_launch_2(grid, threads, smem, st, p, s, a, P, F);
-  else if (v == 3) solve_launch_3(grid, threads, smem, st, p, s, a, P, F);
-  else if (v == 4) solve_launch_4(grid, threads, smem, st, p, s, a, P, F);
-  else solve_launch_5(grid, threads, smem, st, p, s, a, P, F);
+// the per-problem-parameter instantiations (mpc_kernels_tu.cu 9..17)
+cudaError_t solve_set_smem_pp0(int), solve_set_smem_pp1(int), solve_set_smem_pp2(int), solve_set_smem_pp3(int), solve_set_smem_pp4(int), solve_set_smem_pp5(int);
+void solve_launch_pp0(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+void solve_launch_pp1(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+void solve_launch_pp2(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+void solve_launch_pp3(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+void solve_launch_pp4(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+void solve_launch_pp5(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+cudaError_t rollout_set_smem_pp_short(int), rollout_set_smem_pp_general(int), rollout_set_smem_pp_pair(int);
+cudaError_t rollout_occupancy_pp_short(int, int*), rollout_occupancy_pp_general(int, int*), rollout_occupancy_pp_pair(int, int*);
+void rollout_launch_pp_short(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
+void rollout_launch_pp_general(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
+void rollout_launch_pp_pair(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const RolloutArgs&);
+cudaError_t step_set_smem_pp_short(int), step_set_smem_pp_general(int), step_set_smem_pp_pair(int);
+void step_launch_pp_short(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
+void step_launch_pp_general(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
+void step_launch_pp_pair(int, int, cudaStream_t, const Params&, const Settings&, const cudampc_rollout_cfg&, const StepArgs&);
+
+typedef void (*SolveLaunchFn)(int, int, int, cudaStream_t, const Params&, const Settings&, const BatchArgs&, int, int);
+static cudaError_t (*const k_solve_set_smem[2][6])(int) = {
+  {solve_set_smem_0, solve_set_smem_1, solve_set_smem_2, solve_set_smem_3, solve_set_smem_4, solve_set_smem_5},
+  {solve_set_smem_pp0, solve_set_smem_pp1, solve_set_smem_pp2, solve_set_smem_pp3, solve_set_smem_pp4, solve_set_smem_pp5}};
+static const SolveLaunchFn k_solve_launch[2][6] = {
+  {solve_launch_0, solve_launch_1, solve_launch_2, solve_launch_3, solve_launch_4, solve_launch_5},
+  {solve_launch_pp0, solve_launch_pp1, solve_launch_pp2, solve_launch_pp3, solve_launch_pp4, solve_launch_pp5}};
+cudaError_t solve_set_smem(int v, int bytes, bool pp) { return k_solve_set_smem[pp][v < 5 ? v : 5](bytes); }
+void solve_launch(int v, int grid, int threads, int smem, cudaStream_t st, const Params& p, const Settings& s, const BatchArgs& a, int P, int F, bool pp) {
+  k_solve_launch[pp][v < 5 ? v : 5](grid, threads, smem, st, p, s, a, P, F);
 }
-cudaError_t rollout_set_smem(int f, int bytes) { return f == FORM_SHORT ? rollout_set_smem_short(bytes) : f == FORM_PAIR ? rollout_set_smem_pair(bytes) : rollout_set_smem_general(bytes); }
-cudaError_t rollout_occupancy(int f, int bytes, int* n) {
+cudaError_t rollout_set_smem(int f, int bytes, bool pp) {
+  if (pp) return f == FORM_SHORT ? rollout_set_smem_pp_short(bytes) : f == FORM_PAIR ? rollout_set_smem_pp_pair(bytes) : rollout_set_smem_pp_general(bytes);
+  return f == FORM_SHORT ? rollout_set_smem_short(bytes) : f == FORM_PAIR ? rollout_set_smem_pair(bytes) : rollout_set_smem_general(bytes);
+}
+cudaError_t rollout_occupancy(int f, int bytes, int* n, bool pp) {
+  if (pp) return f == FORM_SHORT ? rollout_occupancy_pp_short(bytes, n) : f == FORM_PAIR ? rollout_occupancy_pp_pair(bytes, n) : rollout_occupancy_pp_general(bytes, n);
   return f == FORM_SHORT ? rollout_occupancy_short(bytes, n) : f == FORM_PAIR ? rollout_occupancy_pair(bytes, n) : rollout_occupancy_general(bytes, n);
 }
-void rollout_launch(int f, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const RolloutArgs& a) {
-  if (f == FORM_SHORT) rollout_launch_short(grid, smem, st, p, s, cfg, a);
+void rollout_launch(int f, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const RolloutArgs& a, bool pp) {
+  if (pp) {
+    if (f == FORM_SHORT) rollout_launch_pp_short(grid, smem, st, p, s, cfg, a);
+    else if (f == FORM_PAIR) rollout_launch_pp_pair(grid, smem, st, p, s, cfg, a);
+    else rollout_launch_pp_general(grid, smem, st, p, s, cfg, a);
+  } else if (f == FORM_SHORT) rollout_launch_short(grid, smem, st, p, s, cfg, a);
   else if (f == FORM_PAIR) rollout_launch_pair(grid, smem, st, p, s, cfg, a);
   else rollout_launch_general(grid, smem, st, p, s, cfg, a);
 }
-cudaError_t step_set_smem(int f, int bytes) { return f == FORM_SHORT ? step_set_smem_short(bytes) : f == FORM_PAIR ? step_set_smem_pair(bytes) : step_set_smem_general(bytes); }
-void step_launch(int f, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a) {
-  if (f == FORM_SHORT) step_launch_short(grid, smem, st, p, s, cfg, a);
+cudaError_t step_set_smem(int f, int bytes, bool pp) {
+  if (pp) return f == FORM_SHORT ? step_set_smem_pp_short(bytes) : f == FORM_PAIR ? step_set_smem_pp_pair(bytes) : step_set_smem_pp_general(bytes);
+  return f == FORM_SHORT ? step_set_smem_short(bytes) : f == FORM_PAIR ? step_set_smem_pair(bytes) : step_set_smem_general(bytes);
+}
+void step_launch(int f, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a, bool pp) {
+  if (pp) {
+    if (f == FORM_SHORT) step_launch_pp_short(grid, smem, st, p, s, cfg, a);
+    else if (f == FORM_PAIR) step_launch_pp_pair(grid, smem, st, p, s, cfg, a);
+    else step_launch_pp_general(grid, smem, st, p, s, cfg, a);
+  } else if (f == FORM_SHORT) step_launch_short(grid, smem, st, p, s, cfg, a);
   else if (f == FORM_PAIR) step_launch_pair(grid, smem, st, p, s, cfg, a);
   else step_launch_general(grid, smem, st, p, s, cfg, a);
 }
@@ -249,56 +288,13 @@ static int fail(cudampc_handle* h, int code, const char* fmt, const char* detail
     }                                                                                       \
   } while (0)
 
-// Smallest eigenvalue of the symmetric n x n matrix W (n <= 4), cyclic Jacobi.  cp.quad_form (mpc_controller.py:74-75,112)
-// accepts any PSD matrix; the library accepts exactly those (relative tolerance 1e-12) and rejects indefinite ones.
-static double min_eig_sym(const double* Win, int n, double* scale) {
-  double a[4][4];
-  double mx = 0.0;
-  for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j) { a[i][j] = Win[i * n + j]; if (fabs(a[i][j]) > mx) mx = fabs(a[i][j]); }
-  *scale = mx;
-  for (int sweep = 0; sweep < 50; ++sweep) {
-    double off = 0.0;
-    for (int i = 0; i < n; ++i) for (int j = 0; j < i; ++j) off += a[i][j] * a[i][j];
-    if (off <= 1e-30 * mx * mx) break;
-    for (int p = 0; p < n; ++p)
-      for (int q = p + 1; q < n; ++q) {
-        if (a[p][q] == 0.0) continue;
-        const double th = (a[q][q] - a[p][p]) / (2.0 * a[p][q]);
-        const double t = (th >= 0 ? 1.0 : -1.0) / (fabs(th) + sqrt(th * th + 1.0)), c = 1.0 / sqrt(t * t + 1.0), sn = t * c;
-        for (int k = 0; k < n; ++k) { const double x = a[k][p], y = a[k][q]; a[k][p] = c * x - sn * y; a[k][q] = sn * x + c * y; }
-        for (int k = 0; k < n; ++k) { const double x = a[p][k], y = a[q][k]; a[p][k] = c * x - sn * y; a[q][k] = sn * x + c * y; }
-      }
-  }
-  double mn = a[0][0];
-  for (int i = 1; i < n; ++i) if (a[i][i] < mn) mn = a[i][i];
-  return mn;
-}
-
 static int convert_params(const cudampc_params* in, Params* p, cudampc_handle* h) {
   if (!in) return fail(h, CUDAMPC_ERR_INVALID, "%s", "params is NULL");
-  if (in->horizon < 1 || in->horizon > 256) return fail(h, CUDAMPC_ERR_INVALID, "%s", "horizon must be in [1, 256]");
-  if (!(in->dt > 0.0) || !(in->wheelbase_px > 0.0)) return fail(h, CUDAMPC_ERR_INVALID, "%s", "dt and wheelbase_px must be > 0");
-  p->L = in->wheelbase_px; p->dt = in->dt; p->N = in->horizon;
-  // quad_form(e, W) = e'We = 1/2 e'(W + W')e: the P block of the QP is the symmetric matrix W + W'
-  for (int i = 0; i < 4; ++i)
-    for (int j = 0; j < 4; ++j) { p->pq[i][j] = in->q[4 * i + j] + in->q[4 * j + i]; p->pqn[i][j] = in->q_terminal[4 * i + j] + in->q_terminal[4 * j + i]; }
-  for (int i = 0; i < 2; ++i)
-    for (int j = 0; j < 2; ++j) p->pr[i][j] = in->r[2 * i + j] + in->r[2 * j + i];
-  {
-    double sc;
-    double e = min_eig_sym(&p->pq[0][0], 4, &sc);
-    if (!(sc > 0.0) || !(e >= -1e-12 * sc) || !isfinite(e)) return fail(h, CUDAMPC_ERR_INVALID, "%s", "q must be positive semidefinite and non-zero");
-    e = min_eig_sym(&p->pqn[0][0], 4, &sc);
-    if (!(sc > 0.0) || !(e >= -1e-12 * sc) || !isfinite(e)) return fail(h, CUDAMPC_ERR_INVALID, "%s", "q_terminal must be positive semidefinite and non-zero");
-    e = min_eig_sym(&p->pr[0][0], 2, &sc);
-    if (!(sc > 0.0) || !(e >= -1e-12 * sc) || !isfinite(e)) return fail(h, CUDAMPC_ERR_INVALID, "%s", "r must be positive semidefinite and non-zero");
-  }
-  p->u_lo[0] = in->u_bounds[0]; p->u_hi[0] = in->u_bounds[1]; p->u_lo[1] = in->u_bounds[2]; p->u_hi[1] = in->u_bounds[3];
-  p->v_lo = in->v_bounds[0]; p->v_hi = in->v_bounds[1];
-  p->du_lo[0] = in->du_bounds[0]; p->du_hi[0] = in->du_bounds[1]; p->du_lo[1] = in->du_bounds[2]; p->du_hi[1] = in->du_bounds[3];
-  p->w_v = in->slack_velocity; p->w_u = in->slack_input; p->w_du = in->slack_rate;
-  if (!(p->w_v > 0.0) || !(p->w_u > 0.0) || !(p->w_du > 0.0)) return fail(h, CUDAMPC_ERR_INVALID, "%s", "slack weights must be > 0");
-  return CUDAMPC_OK;
+  static const char* const why[] = {"", "horizon must be in [1, 256]", "dt and wheelbase_px must be > 0",
+                                    "q must be positive semidefinite and non-zero", "q_terminal must be positive semidefinite and non-zero",
+                                    "r must be positive semidefinite and non-zero", "slack weights must be > 0"};
+  const int rc = params_from_c(in, p);
+  return rc == PARAMS_OK ? CUDAMPC_OK : fail(h, CUDAMPC_ERR_INVALID, "%s", why[rc]);
 }
 
 static int convert_settings(const cudampc_settings* in, Settings* s, cudampc_handle* h) {
@@ -321,6 +317,31 @@ static int convert_settings(const cudampc_settings* in, Settings* s, cudampc_han
   s->polish_refine_iter = in->polish_refine_iter; s->warm_start = in->warm_start > 0 ? 1 : 0;   /* < 0: stateless, see solve_batch */
   s->polish_retry = in->polish_retry < 0 ? 0 : in->polish_retry;
   s->early_polish = in->early_polish; s->early_polish_start = in->early_polish_start;
+  return CUDAMPC_OK;
+}
+
+// Launch configuration of the per-problem-parameter kernels (first *_params call on a handle; the caller holds the device).
+// K_solve: the handle's variant with one Params slot per group after the GroupShared array; K_rollout / K_step: the handle's form
+// with the slot after the workspace.  Both at most the shared-parameter counts, which the handle's allocations are sized for.
+static int pp_configure(cudampc_handle* h) {
+  if (h->pp_ready) return CUDAMPC_OK;
+  int optin = 0;
+  CU(h, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+  const int F = footprint(h->N), per = F * (int)sizeof(double) + (int)sizeof(GroupShared) + (int)sizeof(Params);
+  int P = (optin - 64) / per;
+  if (P > h->grp_P) P = h->grp_P;
+  if (P < 1) return fail(h, CUDAMPC_ERR_UNSUPPORTED, "%s", "horizon too long for per-problem parameters in 227 KB of shared memory");
+  const int smem = P * per + 16;
+  CU(h, solve_set_smem(h->variant, smem, true));
+  const int rsmem = h->smem_bytes + (int)sizeof(Params);
+  int occ = 0;
+  CU(h, rollout_set_smem(h->form, rsmem, true));
+  CU(h, step_set_smem(h->form, rsmem, true));
+  CU(h, rollout_occupancy(h->form, rsmem, &occ, true));
+  if (occ < 1) return fail(h, CUDAMPC_ERR_UNSUPPORTED, "%s", "horizon too long for per-vehicle parameters in 227 KB of shared memory");
+  h->pp_P = P; h->pp_smem = smem;
+  h->pp_roll_per_sm = occ < h->roll_per_sm ? occ : h->roll_per_sm; h->pp_roll_smem = rsmem;
+  h->pp_ready = true;
   return CUDAMPC_OK;
 }
 
@@ -516,19 +537,22 @@ int cudampc_f_discrete_batch(cudampc_handle* h, int batch, const double* x_dev, 
   return CUDAMPC_OK;
 }
 
-int cudampc_solve_batch(cudampc_handle* h, int batch, const double* x0_dev, const double* ref_dev,
-                        const double* u_prev_dev, const cudampc_settings* settings, double* u0_dev, double* Xp_dev,
-                        double* Up_dev, int32_t* status_dev, int32_t* iters_dev, double* pri_res_dev,
-                        double* dua_res_dev, int32_t* info_dev, void* stream) {
+// cudampc_solve_batch (params_dev NULL) and cudampc_solve_batch_params
+static int solve_batch_impl(cudampc_handle* h, int batch, const double* x0_dev, const double* ref_dev,
+                            const double* u_prev_dev, const cudampc_settings* settings, const cudampc_params* params_dev,
+                            double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                            double* pri_res_dev, double* dua_res_dev, int32_t* info_dev, void* stream, const char* name) {
   if (!h) return CUDAMPC_ERR_INVALID;
-  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s", "solve_batch: batch out of range for this handle");
+  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s: batch out of range for this handle", name);
   if (!x0_dev || !ref_dev || !u0_dev || !Xp_dev || !Up_dev || !status_dev || !iters_dev)
-    return fail(h, CUDAMPC_ERR_INVALID, "%s", "solve_batch: NULL pointer");
+    return fail(h, CUDAMPC_ERR_INVALID, "%s: NULL pointer", name);
   Settings s;
   int rc = convert_settings(settings, &s, h);
   if (rc) return rc;
   if (batch == 0) return CUDAMPC_OK;
   ON_DEVICE(h);
+  const bool pp = params_dev != nullptr;
+  if (pp && (rc = pp_configure(h))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   CU(h, cudaMemsetAsync(h->counter, 0, sizeof(int), st));
   BatchArgs a;
@@ -537,13 +561,32 @@ int cudampc_solve_batch(cudampc_handle* h, int batch, const double* x0_dev, cons
   a.group_slot0 = h->max_batch;
   a.u0 = u0_dev; a.Xp = Xp_dev; a.Up = Up_dev; a.status = status_dev; a.iters = iters_dev;
   a.pri = pri_res_dev; a.dua = dua_res_dev; a.info = info_dev; a.counter = h->counter; a.batch = batch; a.tags = h->tags;
-  int grid = (batch + h->grp_P - 1) / h->grp_P;
+  a.params = params_dev;
+  const int P = pp ? h->pp_P : h->grp_P;
+  int grid = (batch + P - 1) / P;
   if (grid > h->sms) grid = h->sms;
-  const int threads = 32 * h->grp_wpp * h->grp_P;
-  solve_launch(h->variant, grid, threads, h->grp_smem, st, h->p, s, a, h->grp_P, footprint(h->N));
+  const int threads = 32 * h->grp_wpp * P;
+  solve_launch(h->variant, grid, threads, pp ? h->pp_smem : h->grp_smem, st, h->p, s, a, P, footprint(h->N), pp);
   h->launches++;
   CU(h, cudaGetLastError());
   return CUDAMPC_OK;
+}
+
+int cudampc_solve_batch(cudampc_handle* h, int batch, const double* x0_dev, const double* ref_dev,
+                        const double* u_prev_dev, const cudampc_settings* settings, double* u0_dev, double* Xp_dev,
+                        double* Up_dev, int32_t* status_dev, int32_t* iters_dev, double* pri_res_dev,
+                        double* dua_res_dev, int32_t* info_dev, void* stream) {
+  return solve_batch_impl(h, batch, x0_dev, ref_dev, u_prev_dev, settings, nullptr, u0_dev, Xp_dev, Up_dev, status_dev, iters_dev,
+                          pri_res_dev, dua_res_dev, info_dev, stream, "solve_batch");
+}
+
+int cudampc_solve_batch_params(cudampc_handle* h, int batch, const double* x0_dev, const double* ref_dev,
+                               const double* u_prev_dev, const cudampc_settings* settings, const cudampc_params* params_dev,
+                               double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                               double* pri_res_dev, double* dua_res_dev, int32_t* info_dev, void* stream) {
+  if (h && !params_dev) return fail(h, CUDAMPC_ERR_INVALID, "%s", "solve_batch_params: NULL pointer");
+  return solve_batch_impl(h, batch, x0_dev, ref_dev, u_prev_dev, settings, params_dev, u0_dev, Xp_dev, Up_dev, status_dev, iters_dev,
+                          pri_res_dev, dua_res_dev, info_dev, stream, "solve_batch_params");
 }
 
 static bool is_pinned(const void* p) {
@@ -638,35 +681,95 @@ int cudampc_build_reference_batch(cudampc_handle* h, int batch, const double* pa
   return CUDAMPC_OK;
 }
 
-int cudampc_rollout_batch(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
-                          int ref_stride, const double* state0_dev, const double* goal_dev,
-                          const cudampc_settings* settings, const cudampc_rollout_cfg* cfg, double* states_dev,
-                          double* controls_dev, int32_t* n_steps_dev, int32_t* flags_dev, int32_t* step_status_dev,
-                          int32_t* step_iters_dev, void* stream) {
+// cudampc_rollout_batch (params_dev NULL) and cudampc_rollout_batch_params
+static int rollout_batch_impl(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                              int ref_stride, const double* state0_dev, const double* goal_dev,
+                              const cudampc_settings* settings, const cudampc_rollout_cfg* cfg, const cudampc_params* params_dev,
+                              double* states_dev, double* controls_dev, int32_t* n_steps_dev, int32_t* flags_dev,
+                              int32_t* step_status_dev, int32_t* step_iters_dev, void* stream, const char* name) {
   if (!h) return CUDAMPC_ERR_INVALID;
-  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s", "rollout_batch: batch out of range for this handle");
+  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s: batch out of range for this handle", name);
   if (!ref_global_dev || !ref_len_dev || !state0_dev || !goal_dev || !states_dev || !n_steps_dev || !flags_dev || ref_stride < 1)
-    return fail(h, CUDAMPC_ERR_INVALID, "%s", "rollout_batch: NULL pointer or bad stride");
+    return fail(h, CUDAMPC_ERR_INVALID, "%s: NULL pointer or bad stride", name);
   cudampc_rollout_cfg c;
   if (cfg) c = *cfg; else cudampc_default_rollout_cfg(&c);
-  if (c.sim_steps < 1) return fail(h, CUDAMPC_ERR_INVALID, "%s", "rollout_batch: sim_steps must be >= 1");
+  if (c.sim_steps < 1) return fail(h, CUDAMPC_ERR_INVALID, "%s: sim_steps must be >= 1", name);
   Settings s;
   int rc = convert_settings(settings, &s, h);
   if (rc) return rc;
   if (batch == 0) return CUDAMPC_OK;
   ON_DEVICE(h);
+  const bool pp = params_dev != nullptr;
+  if (pp && (rc = pp_configure(h))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   CU(h, cudaMemsetAsync(h->counter, 0, sizeof(int), st));
   RolloutArgs a;
   a.ref_global = ref_global_dev; a.ref_len = ref_len_dev; a.ref_stride = ref_stride; a.state0 = state0_dev; a.goal = goal_dev;
   a.warm = h->warm; a.scratch = h->scratch; a.fsave = getenv("CUDAMPC_NO_FSAVE") ? nullptr : h->fsave; a.work = h->work;
   a.states = states_dev; a.controls = controls_dev; a.n_steps = n_steps_dev; a.flags = flags_dev;
-  a.step_status = step_status_dev; a.step_iters = step_iters_dev; a.counter = h->counter; a.batch = batch;
+  a.step_status = step_status_dev; a.step_iters = step_iters_dev; a.counter = h->counter; a.batch = batch; a.params = params_dev;
   {
-    int grid = h->sms * h->roll_per_sm;
+    int grid = h->sms * (pp ? h->pp_roll_per_sm : h->roll_per_sm);
     if (grid > batch) grid = batch;
-    rollout_launch(h->form, grid, h->smem_bytes, st, h->p, s, c, a);
+    rollout_launch(h->form, grid, pp ? h->pp_roll_smem : h->smem_bytes, st, h->p, s, c, a, pp);
   }
+  h->launches++;
+  CU(h, cudaGetLastError());
+  return CUDAMPC_OK;
+}
+
+int cudampc_rollout_batch(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                          int ref_stride, const double* state0_dev, const double* goal_dev,
+                          const cudampc_settings* settings, const cudampc_rollout_cfg* cfg, double* states_dev,
+                          double* controls_dev, int32_t* n_steps_dev, int32_t* flags_dev, int32_t* step_status_dev,
+                          int32_t* step_iters_dev, void* stream) {
+  return rollout_batch_impl(h, batch, ref_global_dev, ref_len_dev, ref_stride, state0_dev, goal_dev, settings, cfg, nullptr, states_dev,
+                            controls_dev, n_steps_dev, flags_dev, step_status_dev, step_iters_dev, stream, "rollout_batch");
+}
+
+int cudampc_rollout_batch_params(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                                 int ref_stride, const double* state0_dev, const double* goal_dev,
+                                 const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                                 const cudampc_params* params_dev, double* states_dev, double* controls_dev,
+                                 int32_t* n_steps_dev, int32_t* flags_dev, int32_t* step_status_dev, int32_t* step_iters_dev,
+                                 void* stream) {
+  if (h && !params_dev) return fail(h, CUDAMPC_ERR_INVALID, "%s", "rollout_batch_params: NULL pointer or bad stride");
+  return rollout_batch_impl(h, batch, ref_global_dev, ref_len_dev, ref_stride, state0_dev, goal_dev, settings, cfg, params_dev, states_dev,
+                            controls_dev, n_steps_dev, flags_dev, step_status_dev, step_iters_dev, stream, "rollout_batch_params");
+}
+
+// cudampc_track_step_batch (params_dev NULL) and cudampc_track_step_batch_params
+static int track_step_impl(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                           int ref_stride, const double* goal_dev, const double* state_dev,
+                           const cudampc_settings* settings, const cudampc_rollout_cfg* cfg, const cudampc_params* params_dev,
+                           int32_t* path_idx_dev, double* u_prev_dev, int32_t* n_steps_dev, int32_t* flags_dev,
+                           double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
+                           void* stream, const char* name) {
+  if (!h) return CUDAMPC_ERR_INVALID;
+  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s: batch out of range for this handle", name);
+  if (!ref_global_dev || !ref_len_dev || !goal_dev || !state_dev || !path_idx_dev || !u_prev_dev || !n_steps_dev || !flags_dev ||
+      !u0_dev || !status_dev || !iters_dev || ref_stride < 1)
+    return fail(h, CUDAMPC_ERR_INVALID, "%s: NULL pointer or bad stride", name);
+  cudampc_rollout_cfg c;
+  if (cfg) c = *cfg; else cudampc_default_rollout_cfg(&c);
+  Settings s;
+  int rc = convert_settings(settings, &s, h);
+  if (rc) return rc;
+  if (batch == 0) return CUDAMPC_OK;
+  ON_DEVICE(h);
+  const bool pp = params_dev != nullptr;
+  if (pp && (rc = pp_configure(h))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(h, cudaMemsetAsync(h->counter, 0, sizeof(int), st));
+  StepArgs a;
+  a.ref_global = ref_global_dev; a.ref_len = ref_len_dev; a.ref_stride = ref_stride; a.goal = goal_dev; a.state = state_dev;
+  a.warm = h->warm; a.scratch = h->scratch; a.fsave = getenv("CUDAMPC_NO_FSAVE") ? nullptr : h->fsave; a.work = h->work;
+  a.path_idx = path_idx_dev; a.u_prev = u_prev_dev; a.n_steps = n_steps_dev; a.flags = flags_dev;
+  a.u0 = u0_dev; a.Xp = Xp_dev; a.Up = Up_dev; a.status = status_dev; a.iters = iters_dev; a.counter = h->counter; a.batch = batch;
+  a.params = params_dev;
+  int grid = h->sms * (pp ? h->pp_roll_per_sm : h->roll_per_sm);
+  if (grid > batch) grid = batch;
+  step_launch(h->form, grid, pp ? h->pp_roll_smem : h->smem_bytes, st, h->p, s, c, a, pp);
   h->launches++;
   CU(h, cudaGetLastError());
   return CUDAMPC_OK;
@@ -678,31 +781,19 @@ int cudampc_track_step_batch(cudampc_handle* h, int batch, const double* ref_glo
                              int32_t* path_idx_dev, double* u_prev_dev, int32_t* n_steps_dev, int32_t* flags_dev,
                              double* u0_dev, double* Xp_dev, double* Up_dev, int32_t* status_dev, int32_t* iters_dev,
                              void* stream) {
-  if (!h) return CUDAMPC_ERR_INVALID;
-  if (batch < 0 || batch > h->max_batch) return fail(h, CUDAMPC_ERR_INVALID, "%s", "track_step_batch: batch out of range for this handle");
-  if (!ref_global_dev || !ref_len_dev || !goal_dev || !state_dev || !path_idx_dev || !u_prev_dev || !n_steps_dev || !flags_dev ||
-      !u0_dev || !status_dev || !iters_dev || ref_stride < 1)
-    return fail(h, CUDAMPC_ERR_INVALID, "%s", "track_step_batch: NULL pointer or bad stride");
-  cudampc_rollout_cfg c;
-  if (cfg) c = *cfg; else cudampc_default_rollout_cfg(&c);
-  Settings s;
-  int rc = convert_settings(settings, &s, h);
-  if (rc) return rc;
-  if (batch == 0) return CUDAMPC_OK;
-  ON_DEVICE(h);
-  cudaStream_t st = (cudaStream_t)stream;
-  CU(h, cudaMemsetAsync(h->counter, 0, sizeof(int), st));
-  StepArgs a;
-  a.ref_global = ref_global_dev; a.ref_len = ref_len_dev; a.ref_stride = ref_stride; a.goal = goal_dev; a.state = state_dev;
-  a.warm = h->warm; a.scratch = h->scratch; a.fsave = getenv("CUDAMPC_NO_FSAVE") ? nullptr : h->fsave; a.work = h->work;
-  a.path_idx = path_idx_dev; a.u_prev = u_prev_dev; a.n_steps = n_steps_dev; a.flags = flags_dev;
-  a.u0 = u0_dev; a.Xp = Xp_dev; a.Up = Up_dev; a.status = status_dev; a.iters = iters_dev; a.counter = h->counter; a.batch = batch;
-  int grid = h->sms * h->roll_per_sm;
-  if (grid > batch) grid = batch;
-  step_launch(h->form, grid, h->smem_bytes, st, h->p, s, c, a);
-  h->launches++;
-  CU(h, cudaGetLastError());
-  return CUDAMPC_OK;
+  return track_step_impl(h, batch, ref_global_dev, ref_len_dev, ref_stride, goal_dev, state_dev, settings, cfg, nullptr, path_idx_dev,
+                         u_prev_dev, n_steps_dev, flags_dev, u0_dev, Xp_dev, Up_dev, status_dev, iters_dev, stream, "track_step_batch");
+}
+
+int cudampc_track_step_batch_params(cudampc_handle* h, int batch, const double* ref_global_dev, const int32_t* ref_len_dev,
+                                    int ref_stride, const double* goal_dev, const double* state_dev,
+                                    const cudampc_settings* settings, const cudampc_rollout_cfg* cfg,
+                                    const cudampc_params* params_dev, int32_t* path_idx_dev, double* u_prev_dev,
+                                    int32_t* n_steps_dev, int32_t* flags_dev, double* u0_dev, double* Xp_dev, double* Up_dev,
+                                    int32_t* status_dev, int32_t* iters_dev, void* stream) {
+  if (h && !params_dev) return fail(h, CUDAMPC_ERR_INVALID, "%s", "track_step_batch_params: NULL pointer or bad stride");
+  return track_step_impl(h, batch, ref_global_dev, ref_len_dev, ref_stride, goal_dev, state_dev, settings, cfg, params_dev, path_idx_dev,
+                         u_prev_dev, n_steps_dev, flags_dev, u0_dev, Xp_dev, Up_dev, status_dev, iters_dev, stream, "track_step_batch_params");
 }
 
 // dev tool (tools/tag_times.py, libraries built with -DMPC_TIMING): cycles between the driver's tags, summed over a launch

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include "../../include/cudampc.h"
 #include "mpc_exec.cuh"
+#include "mpc_params.h"
 
 using namespace mpc;
 
@@ -17,13 +18,40 @@ struct BatchArgs {
   int group_state;             // 1: stateless solve - the iterate back-ups (warm, scratch) use the resident group's slot, not the problem's
   int group_slot0;             // first of the per-group slots (behind the per-problem ones)
   unsigned long long* tags;    // dev builds only (MPC_TIMING)
+  const cudampc_params* params;  // per-problem kernels (PP): batch records, problem order
 };
+
+// ------------------------------------------------------------------------------------------------
+// Per-problem parameters (the PP instantiations).  Each problem / vehicle b reads its own record params[b]: one lane runs the
+// rules of mpc_params.h on it into the group's Params slot in shared memory, and the group syncs before reading the slot.  A
+// record the rules reject, or whose horizon or dt differs from the launch's (the workspace layout and the time grid of the
+// register-form block are the launch's), leaves slot->N = 0.  Such a problem is not solved.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void load_params(const cudampc_params* rows, int b, const Params& launch, Params* slot) {
+  const cudampc_params* in = rows + b;
+  if (params_from_c(in, slot) != PARAMS_OK || in->horizon != launch.N || !(in->dt == launch.dt)) slot->N = 0;
+}
+// Outputs of a problem whose record is invalid: status CUDAMPC_INVALID_PARAMS, iters 0, NaN u0 / Xp / Up / pri / dua, info 0.
+// The warm-start slot is not touched.
+template <class Exec>
+__device__ __forceinline__ void invalid_problem(Exec& ex, const ProblemIO& io, int N) {
+  const double nan_ = __longlong_as_double(0x7ff8000000000000LL);
+  ex.stages(4 * (N + 1), [&](int i) { io.Xp[i] = nan_; });
+  ex.stages(2 * N, [&](int i) { io.Up[i] = nan_; });
+  ex.single([&]() {
+    io.u0[0] = nan_; io.u0[1] = nan_; *io.status = CUDAMPC_INVALID_PARAMS; *io.iters = 0;
+    if (io.pri_res) *io.pri_res = nan_;
+    if (io.dua_res) *io.dua_res = nan_;
+    if (io.info) for (int i = 0; i < 4; ++i) io.info[i] = 0;
+  });
+}
 
 // ------------------------------------------------------------------------------------------------
 // K_solve: batched MPCController.solve.  The CTA holds P problems, each owned by a group of WPP warps (GroupExec).
 // <256,1>: P <= 8 one-warp groups, 255 registers; <128,2>: P <= 2 two-warp groups for long horizons.
+// PP: per-problem parameters; the P Params slots follow the GroupShared array.
 // ------------------------------------------------------------------------------------------------
-template <int MAXT, int WPP, int FORM>
+template <int MAXT, int WPP, int FORM, bool PP>
 __global__ void __launch_bounds__(MAXT, 1) mpc_solve_kernel(Params p, Settings s, BatchArgs a, int P, int F) {
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -51,7 +79,15 @@ __global__ void __launch_bounds__(MAXT, 1) mpc_solve_kernel(Params p, Settings s
     io.status = a.status + b; io.iters = a.iters + b;
     io.pri_res = a.pri ? a.pri + b : nullptr; io.dua_res = a.dua ? a.dua + b : nullptr;
     io.info = a.info ? a.info + 4 * (size_t)b : nullptr;
-    solve_problem<FORM>(ex, w, p, s, io);
+    if constexpr (PP) {
+      Params* pb = reinterpret_cast<Params*>(reinterpret_cast<GroupShared*>(smem + (size_t)P * F) + P) + warp / WPP;
+      if (ex.gl() == 0) load_params(a.params, b, p, pb);
+      ex.group_sync();
+      if (pb->N == 0) invalid_problem(ex, io, N);
+      else solve_problem<FORM>(ex, w, *pb, s, io);
+    } else {
+      solve_problem<FORM>(ex, w, p, s, io);
+    }
     ex.group_sync();
   }
 }
@@ -120,7 +156,7 @@ __device__ __forceinline__ void reg_drv_finish(RegCtx c, int b) {
   drv_finish(ex, w, io, d);
   ex.group_sync();
 }
-template <int MAXT, int STATE, int WPP>
+template <int MAXT, int STATE, int WPP, bool PP>
 __global__ void __launch_bounds__(MAXT, 1) mpc_solve_reg_kernel(const __grid_constant__ Params p, const __grid_constant__ Settings s,
                                                                 const __grid_constant__ BatchArgs a, int P, int F) {
   extern __shared__ double smem[];
@@ -137,9 +173,18 @@ __global__ void __launch_bounds__(MAXT, 1) mpc_solve_reg_kernel(const __grid_con
   unsigned long long* tg = nullptr;
 #endif
   for (int b = ex.fetch(a.counter); b < a.batch; b = ex.fetch(a.counter)) {
+    const int group = (int)blockIdx.x * P + warp / WPP;
+    const Params* pc = &p;
+    if constexpr (PP) {     // the pieces read the problem's slot; the iteration block keeps the launch's dt
+      Params* pb = reinterpret_cast<Params*>(reinterpret_cast<GroupShared*>(smem + (size_t)P * F) + P) + warp / WPP;
+      if (ex.gl() == 0) load_params(a.params, b, p, pb);
+      ex.group_sync();
+      if (pb->N == 0) { invalid_problem(ex, batch_io(a, b, N, group), N); continue; }
+      pc = pb;
+    }
     // The pieces of the driver are inlined; none of their values is alive across a block (Drv lives in shared memory
     // between them).
-    const RegCtx c{&p, &s, &a, base, sh, N, fpad, xpad, lane, warp, (int)blockIdx.x * P + warp / WPP};
+    const RegCtx c{pc, &s, &a, base, sh, N, fpad, xpad, lane, warp, group};
     reg_drv_begin<WPP>(c, b);
     while (!*(volatile int*)&sh->drv.finished) {
       if (*(volatile int*)&sh->drv.phase == PH_ADMM) {       // else a polish pass ran its solves: its residuals are next
@@ -170,6 +215,7 @@ struct RolloutArgs {
   double* warm; double* scratch; double* fsave; double* work;   // fsave: oe_doubles(N) per CTA, or null; work: per vehicle 16 doubles (state, u_prev, u0 out) + Xp/Up scratch
   double* states; double* controls; int* n_steps; int* flags; int* step_status; int* step_iters;
   int* counter; int batch;
+  const cudampc_params* params;  // per-vehicle kernels (PP): batch records, vehicle order
 };
 
 __device__ __forceinline__ void f_discrete_dev(const Params& p, const double* x, const double* u, double* out) {
@@ -180,7 +226,9 @@ __device__ __forceinline__ void f_discrete_dev(const Params& p, const double* x,
 // (a) The solve of the step (_solve_with_relaxation, control_stage.py:45-56,126-129): window at path_idx with tail padding,
 // warm start from the problem's slot once the vehicle has stepped, one cold retry with v_ref * relax_v_scale and widened
 // du_bounds on failure (sets flags bit 2).  io carries everything but the window.  Returns the final status.
-template <int FORM, class Exec>
+// PP: p is the vehicle's Params slot in shared memory; the retry widens the slot's own du_bounds and restores them afterwards
+// (a copy of the slot would take 416 bytes of local memory in every lane).
+template <int FORM, bool PP, class Exec>
 __device__ __forceinline__ int track_solve(Exec& ex, const View& w, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg,
                                            ProblemIO io, const double* refg, int path_idx, int len, bool stepped, int& flags) {
   io.ref = RefWin{refg, path_idx, len, 1.0};
@@ -190,13 +238,25 @@ __device__ __forceinline__ int track_solve(Exec& ex, const View& w, const Params
   ex.group_sync();
   int status = *io.status;
   if (status != STATUS_SOLVED && status != STATUS_SOLVED_INACCURATE && cfg.relax_on_failure) {
-    Params pr = p;
-    pr.du_lo[0] -= cfg.relax_da; pr.du_hi[0] += cfg.relax_da;
-    pr.du_lo[1] -= cfg.relax_ddelta; pr.du_hi[1] += cfg.relax_ddelta;
     io.ref.vscale = cfg.relax_v_scale;
     ss.warm_start = 0;
-    solve_problem<FORM>(ex, w, pr, ss, io);
-    ex.group_sync();
+    if constexpr (PP) {
+      Params& pr = const_cast<Params&>(p);
+      const double lo0 = pr.du_lo[0], hi0 = pr.du_hi[0], lo1 = pr.du_lo[1], hi1 = pr.du_hi[1];
+      ex.single([&]() {
+        pr.du_lo[0] -= cfg.relax_da; pr.du_hi[0] += cfg.relax_da;
+        pr.du_lo[1] -= cfg.relax_ddelta; pr.du_hi[1] += cfg.relax_ddelta;
+      });
+      solve_problem<FORM>(ex, w, pr, ss, io);
+      ex.group_sync();
+      ex.single([&]() { pr.du_lo[0] = lo0; pr.du_hi[0] = hi0; pr.du_lo[1] = lo1; pr.du_hi[1] = hi1; });
+    } else {
+      Params pr = p;
+      pr.du_lo[0] -= cfg.relax_da; pr.du_hi[0] += cfg.relax_da;
+      pr.du_lo[1] -= cfg.relax_ddelta; pr.du_hi[1] += cfg.relax_ddelta;
+      solve_problem<FORM>(ex, w, pr, ss, io);
+      ex.group_sync();
+    }
     status = *io.status;
     flags |= 4;
   }
@@ -214,8 +274,20 @@ __device__ __forceinline__ bool track_advance(const cudampc_rollout_cfg& cfg, co
   return hypot(x[0] - goal[0], x[1] - goal[1]) < cfg.goal_radius;
 }
 
+// A vehicle that takes no step: NaN states / controls, zero step status / iters, n_steps 0
+template <class Exec>
+__device__ __forceinline__ void stopped_vehicle(Exec& ex, const cudampc_rollout_cfg& cfg, const RolloutArgs& a, int b, int flags) {
+  const double nan_ = __longlong_as_double(0x7ff8000000000000LL);
+  const int T0 = cfg.sim_steps;
+  ex.stages(T0 * 4, [&](int i) { a.states[(size_t)T0 * b * 4 + i] = nan_; });
+  if (a.controls) ex.stages(T0 * 2, [&](int i) { a.controls[(size_t)T0 * b * 2 + i] = nan_; });
+  if (a.step_status) ex.stages(T0, [&](int i) { a.step_status[(size_t)T0 * b + i] = 0; });
+  if (a.step_iters) ex.stages(T0, [&](int i) { a.step_iters[(size_t)T0 * b + i] = 0; });
+  ex.single([&]() { a.n_steps[b] = 0; a.flags[b] = flags; });
+}
+
 // One vehicle, all steps (TrajectoryTracker.track loop body, control_stage.py:100-150), generic in the execution policy
-template <int FORM, class Exec>
+template <int FORM, bool PP, class Exec>
 __device__ __forceinline__ void rollout_vehicle(Exec& ex, const View& w, const Params& p, const Settings& s,
                                                 const cudampc_rollout_cfg& cfg, const RolloutArgs& a, int b) {
   const int N = p.N;
@@ -226,12 +298,7 @@ __device__ __forceinline__ void rollout_vehicle(Exec& ex, const View& w, const P
   const double* refg = a.ref_global + (size_t)4 * a.ref_stride * b;
   const int len = a.ref_len[b];
   if (len < 1) {                                           // control_stage.py:71-72 raises for an empty path; per vehicle: aborted, no steps
-    const int T0 = cfg.sim_steps;
-    ex.stages(T0 * 4, [&](int i) { a.states[(size_t)T0 * b * 4 + i] = nan_; });
-    if (a.controls) ex.stages(T0 * 2, [&](int i) { a.controls[(size_t)T0 * b * 2 + i] = nan_; });
-    if (a.step_status) ex.stages(T0, [&](int i) { a.step_status[(size_t)T0 * b + i] = 0; });
-    if (a.step_iters) ex.stages(T0, [&](int i) { a.step_iters[(size_t)T0 * b + i] = 0; });
-    ex.single([&]() { a.n_steps[b] = 0; a.flags[b] = 2; });
+    stopped_vehicle(ex, cfg, a, b, 2);
     return;
   }
   ex.single([&]() {
@@ -250,7 +317,7 @@ __device__ __forceinline__ void rollout_vehicle(Exec& ex, const View& w, const P
     io.fsave = a.fsave ? a.fsave + (size_t)oe_doubles(N) * blockIdx.x : nullptr;
     io.u0 = wkb + 6; io.Xp = wkb + 16; io.Up = wkb + 16 + 4 * (N + 1);
     io.status = st_out; io.iters = it_out; io.pri_res = nullptr; io.dua_res = nullptr; io.info = nullptr;
-    const int status = track_solve<FORM>(ex, w, p, s, cfg, io, refg, path_idx, len, step > 0, flags);
+    const int status = track_solve<FORM, PP>(ex, w, p, s, cfg, io, refg, path_idx, len, step > 0, flags);
     if (status != STATUS_SOLVED && status != STATUS_SOLVED_INACCURATE) { flags |= 2; break; }
     // integrate, carry u_prev, path index rule, goal test (control_stage.py:127-150)
     double xn[4];
@@ -280,14 +347,26 @@ __device__ __forceinline__ void rollout_vehicle(Exec& ex, const View& w, const P
   ex.single([&]() { a.n_steps[b] = nst; a.flags[b] = flags; });
 }
 
-template <int FORM>
+// PP: per-vehicle parameters, the Params slot follows the workspace.  A vehicle with an invalid record takes no step and is
+// flagged aborted (bit 1) with invalid parameters (bit 3).
+template <int FORM, bool PP>
 __global__ void __launch_bounds__(32) mpc_rollout_kernel(Params p, Settings s, cudampc_rollout_cfg cfg, RolloutArgs a) {
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31;
   int fpad, xpad; layout_pads(p.N, fpad, xpad);
   View w{smem, p.N, fpad, xpad};
   GroupExec<1> ex{lane, 0, nullptr};
-  for (int b = ex.fetch(a.counter); b < a.batch; b = ex.fetch(a.counter)) rollout_vehicle<FORM>(ex, w, p, s, cfg, a, b);
+  for (int b = ex.fetch(a.counter); b < a.batch; b = ex.fetch(a.counter)) {
+    if constexpr (PP) {
+      Params* pb = reinterpret_cast<Params*>(smem + footprint(p.N));
+      if (lane == 0) load_params(a.params, b, p, pb);
+      __syncwarp();
+      if (pb->N == 0) stopped_vehicle(ex, cfg, a, b, 2 | 8);
+      else rollout_vehicle<FORM, true>(ex, w, *pb, s, cfg, a, b);
+    } else {
+      rollout_vehicle<FORM, false>(ex, w, p, s, cfg, a, b);
+    }
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -302,11 +381,13 @@ struct StepArgs {
   int* path_idx; double* u_prev; int* n_steps; int* flags;
   double* u0; double* Xp; double* Up; int* status; int* iters;
   int* counter; int batch;
+  const cudampc_params* params;  // per-vehicle kernels (PP): batch records, vehicle order
 };
 
-template <int FORM, class Exec>
+// bad (PP only): the vehicle's record is invalid; it is flagged aborted (bit 1) with invalid parameters (bit 3) and solves nothing
+template <int FORM, bool PP, class Exec>
 __device__ __forceinline__ void step_vehicle(Exec& ex, const View& w, const Params& p, const Settings& s,
-                                             const cudampc_rollout_cfg& cfg, const StepArgs& a, int b) {
+                                             const cudampc_rollout_cfg& cfg, const StepArgs& a, int b, bool bad) {
   const int N = p.N;
   const int ws = warm_size(N);
   const int wk = 16 + 4 * (N + 1) + 2 * N;
@@ -318,8 +399,14 @@ __device__ __forceinline__ void step_vehicle(Exec& ex, const View& w, const Para
   const int len = a.ref_len[b];
   const int stepped = a.n_steps[b] > 0;
   int flags = a.flags[b], path_idx = a.path_idx[b];
-  if (len < 1) flags = 2;                                  // empty path: aborted, no solve (as K_rollout)
-  else if (!(flags & 3) && stepped && track_advance(cfg, refg, len, a.goal + 2 * (size_t)b, a.state + 4 * (size_t)b, path_idx)) flags |= 1;
+  if constexpr (PP) {
+    if (len < 1) flags = bad ? 2 | 8 : 2;
+    else if (bad) flags |= 2 | 8;
+    else if (!(flags & 3) && stepped && track_advance(cfg, refg, len, a.goal + 2 * (size_t)b, a.state + 4 * (size_t)b, path_idx)) flags |= 1;
+  } else {
+    if (len < 1) flags = 2;                                // empty path: aborted, no solve (as K_rollout)
+    else if (!(flags & 3) && stepped && track_advance(cfg, refg, len, a.goal + 2 * (size_t)b, a.state + 4 * (size_t)b, path_idx)) flags |= 1;
+  }
   double* Xp = a.Xp ? a.Xp + (size_t)4 * (N + 1) * b : wkb + 16;
   double* Up = a.Up ? a.Up + (size_t)2 * N * b : wkb + 16 + 4 * (N + 1);
   if (!(flags & 3)) {
@@ -333,7 +420,7 @@ __device__ __forceinline__ void step_vehicle(Exec& ex, const View& w, const Para
     io.fsave = a.fsave ? a.fsave + (size_t)oe_doubles(N) * blockIdx.x : nullptr;
     io.u0 = wkb + 6; io.Xp = Xp; io.Up = Up;
     io.status = a.status + b; io.iters = a.iters + b; io.pri_res = nullptr; io.dua_res = nullptr; io.info = nullptr;
-    const int status = track_solve<FORM>(ex, w, p, s, cfg, io, refg, path_idx, len, stepped, flags);
+    const int status = track_solve<FORM, PP>(ex, w, p, s, cfg, io, refg, path_idx, len, stepped, flags);
     if (status == STATUS_SOLVED || status == STATUS_SOLVED_INACCURATE) {
       ex.single([&]() {
         a.u0[2 * (size_t)b] = wkb[6]; a.u0[2 * (size_t)b + 1] = wkb[7];
@@ -352,14 +439,29 @@ __device__ __forceinline__ void step_vehicle(Exec& ex, const View& w, const Para
   ex.single([&]() { a.u0[2 * (size_t)b] = nan_; a.u0[2 * (size_t)b + 1] = nan_; a.path_idx[b] = path_idx; a.flags[b] = flags; });
 }
 
-template <int FORM>
+// PP: as K_rollout; an invalid vehicle's slot gets the launch's horizon (the sizes of its NaN outputs), and bad = true stops it
+template <int FORM, bool PP>
 __global__ void __launch_bounds__(32) mpc_track_step_kernel(Params p, Settings s, cudampc_rollout_cfg cfg, StepArgs a) {
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31;
   int fpad, xpad; layout_pads(p.N, fpad, xpad);
   View w{smem, p.N, fpad, xpad};
   GroupExec<1> ex{lane, 0, nullptr};
-  for (int b = ex.fetch(a.counter); b < a.batch; b = ex.fetch(a.counter)) step_vehicle<FORM>(ex, w, p, s, cfg, a, b);
+  for (int b = ex.fetch(a.counter); b < a.batch; b = ex.fetch(a.counter)) {
+    if constexpr (PP) {
+      Params* pb = reinterpret_cast<Params*>(smem + footprint(p.N));
+      int bad = 0;
+      if (lane == 0) {
+        load_params(a.params, b, p, pb);
+        bad = pb->N == 0;
+        if (bad) pb->N = p.N;
+      }
+      bad = __shfl_sync(0xffffffffu, bad, 0);
+      step_vehicle<FORM, true>(ex, w, *pb, s, cfg, a, b, bad != 0);
+    } else {
+      step_vehicle<FORM, false>(ex, w, p, s, cfg, a, b, false);
+    }
+  }
 }
 
 
@@ -370,10 +472,11 @@ __global__ void __launch_bounds__(32) mpc_track_step_kernel(Params p, Settings s
 // problem (general form, long horizons); K_rollout and K_step: one warp per vehicle, any of the three forms (mpc_solve.h FORM_*),
 // both in the rollout's translation unit of that form.
 enum SolveVariant { SOLVE_W1_SHORT = 0, SOLVE_W1 = 1, SOLVE_W2 = 2, SOLVE_W1_PAIR = 3, SOLVE_W2_REG = 4, SOLVE_W1_REG = 5 };
-cudaError_t solve_set_smem(int variant, int bytes);
-void solve_launch(int variant, int grid, int threads, int smem, cudaStream_t st, const Params& p, const Settings& s, const BatchArgs& a, int P, int F);
-cudaError_t rollout_set_smem(int form, int bytes);
-cudaError_t rollout_occupancy(int form, int bytes, int* blocks_per_sm);
-void rollout_launch(int form, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const RolloutArgs& a);
-cudaError_t step_set_smem(int form, int bytes);
-void step_launch(int form, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a);
+// pp: the per-problem-parameter instantiation of the same variant / form
+cudaError_t solve_set_smem(int variant, int bytes, bool pp = false);
+void solve_launch(int variant, int grid, int threads, int smem, cudaStream_t st, const Params& p, const Settings& s, const BatchArgs& a, int P, int F, bool pp = false);
+cudaError_t rollout_set_smem(int form, int bytes, bool pp = false);
+cudaError_t rollout_occupancy(int form, int bytes, int* blocks_per_sm, bool pp = false);
+void rollout_launch(int form, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const RolloutArgs& a, bool pp = false);
+cudaError_t step_set_smem(int form, int bytes, bool pp = false);
+void step_launch(int form, int grid, int smem, cudaStream_t st, const Params& p, const Settings& s, const cudampc_rollout_cfg& cfg, const StepArgs& a, bool pp = false);

@@ -7,8 +7,9 @@ Same names, arguments and failure behaviour as /root/reference/src/control/mpc_c
   ``(u0 (2,), Xp (4,N+1), Up (2,N))`` or ``(None, None, None)`` when the solver status is not
   optimal / optimal_inaccurate (mpc_controller.py:137-141); inputs are not mutated; ``u_init`` is
   accepted and ignored exactly as upstream (mpc_controller.py:50-51 computes it and never uses it);
-* new: ``solve_batch`` (thousands of independent problems per launch), ``linearize_batch`` and solver
-  settings as constructor arguments (upstream hard-codes them, mpc_controller.py:121-131).
+* new: ``solve_batch`` (thousands of independent problems per launch, optionally each with its own
+  ``MPCParameters``), ``linearize_batch`` and solver settings as constructor arguments (upstream hard-codes them,
+  mpc_controller.py:121-131).
 """
 from __future__ import annotations
 
@@ -104,6 +105,51 @@ def params_to_c(p: MPCParameters) -> _lib.Params:
     c.du_bounds[:] = [p.du_bounds[0][0], p.du_bounds[0][1], p.du_bounds[1][0], p.du_bounds[1][1]]
     c.slack_velocity, c.slack_input, c.slack_rate = float(p.slack_velocity), float(p.slack_input), float(p.slack_rate)
     return c
+
+
+def params_array(params) -> np.ndarray:
+    """One ``_lib.PARAMS_DTYPE`` record (the layout of ``cudampc_params``) per ``MPCParameters`` of the sequence ``params``.
+    The array can be edited field-wise for sweeps (``arr["du_bounds"][:, 3] = ...``) and passed as ``params=`` /
+    ``vehicle_params=``."""
+    return np.frombuffer(b"".join(bytes(params_to_c(p)) for p in params), dtype=_lib.PARAMS_DTYPE).copy()
+
+
+def params_rows(params, batch: int, base: MPCParameters):
+    """Per-problem parameters checked against a handle created with ``base``: a ``PARAMS_DTYPE`` array of ``batch`` records for
+    a sequence of ``MPCParameters`` or such an array, or the CUDA ``uint8`` tensor ``(batch, PARAMS_DTYPE.itemsize)`` as given.
+    Raises ``ValueError`` for a wrong shape, or a record whose horizon or dt differs from ``base`` (dt compared exactly); the
+    other rules are applied per record on the device (a rejected record gets ``STATUS_INVALID_PARAMS``).  The horizon and dt of
+    a tensor's records are checked there too."""
+    rec = _lib.PARAMS_DTYPE.itemsize
+    if hasattr(params, "is_cuda"):
+        import torch
+        if tuple(params.shape) != (batch, rec) or params.dtype != torch.uint8 or not params.is_cuda or not params.is_contiguous():
+            raise ValueError(f"params: expected a contiguous CUDA uint8 tensor of shape ({batch}, {rec}); "
+                             f"got {params.dtype} {tuple(params.shape)} on {params.device}")
+        return params
+    if isinstance(params, np.ndarray) and params.dtype == _lib.PARAMS_DTYPE:
+        arr = np.ascontiguousarray(params)
+    elif isinstance(params, np.ndarray):
+        raise ValueError(f"params: expected an array of dtype PARAMS_DTYPE or a sequence of MPCParameters; got dtype {params.dtype}")
+    else:
+        arr = params_array(params)
+    if arr.shape != (batch,):
+        raise ValueError(f"params: expected {batch} records; got shape {arr.shape}")
+    bad = np.flatnonzero((arr["horizon"] != int(base.horizon)) | (arr["dt"] != float(base.dt)))
+    if bad.size:
+        raise ValueError(f"params: horizon and dt must equal the controller's ({base.horizon}, {base.dt!r}); "
+                         f"records {bad[:8].tolist()} differ")
+    return arr
+
+
+def params_to_device(rows, device):
+    """``params_rows`` output as the CUDA uint8 tensor the *_params entry points read."""
+    import torch
+    if hasattr(rows, "is_cuda"):
+        if rows.device != device:
+            raise ValueError(f"params live on {rows.device}; expected {device}")
+        return rows
+    return torch.from_numpy(rows.view(np.uint8).reshape(len(rows), _lib.PARAMS_DTYPE.itemsize)).to(device)
 
 
 @dataclass
@@ -213,13 +259,19 @@ class MPCController:
         return res.u0[0].copy(), res.Xp[0].copy(), res.Up[0].copy()
 
     # -- batched entry points -------------------------------------------------------------------
-    def solve_batch(self, x0, ref, *, u_prev=None, settings: Optional[SolverSettings] = None, stream=None) -> BatchResult:
+    def solve_batch(self, x0, ref, *, u_prev=None, settings: Optional[SolverSettings] = None, stream=None, params=None) -> BatchResult:
         """``x0 (B,4)``, ``ref (B,N+1,4)``, ``u_prev (B,2)|None`` as NumPy arrays (host path: pinned staging,
-        H2D, solve, D2H) or as torch CUDA fp64 tensors (device path: asynchronous on the current stream)."""
+        H2D, solve, D2H) or as torch CUDA fp64 tensors (device path: asynchronous on the current stream).
+
+        ``params``: per-problem parameters, problem b solved with its own record (``params_rows``: a sequence of
+        ``MPCParameters``, a ``PARAMS_DTYPE`` array or a CUDA uint8 tensor ``(B, 416)``; horizon and dt as this controller's).
+        With NumPy inputs the call then stages through device tensors and synchronises.  A record the parameter rules reject
+        gets status ``STATUS_INVALID_PARAMS`` and NaN outputs."""
         s = (settings or self.settings).to_c()
         N = self._params.horizon
         if _is_torch_cuda(x0):
-            return self._solve_batch_device(x0, ref, u_prev, s, stream)
+            rows = None if params is None else params_rows(params, x0.shape[0], self._params)
+            return self._solve_batch_device(x0, ref, u_prev, s, stream, rows)
         x0 = np.ascontiguousarray(x0, dtype=np.float64)
         ref = np.ascontiguousarray(ref, dtype=np.float64)
         B = x0.shape[0]
@@ -230,6 +282,14 @@ class MPCController:
             up = np.ascontiguousarray(u_prev, dtype=np.float64)
             if up.shape != (B, 2):
                 raise ValueError(f"expected u_prev (B,2); got {up.shape}")
+        if params is not None:
+            rows = params_rows(params, B, self._params)
+            import torch
+            dev = torch.device("cuda", self._device)
+            t = lambda a: None if a is None else torch.as_tensor(a).to(dev)
+            res = self._solve_batch_device(t(x0), t(ref), t(up), s, None, rows)
+            torch.cuda.synchronize(dev)
+            return BatchResult(*(x.cpu().numpy() for x in (res.u0, res.Xp, res.Up, res.status, res.iters, res.pri_res, res.dua_res, res.info)))
         out = self._host_outputs(B, N)
         if B == 0:
             return out
@@ -255,7 +315,7 @@ class MPCController:
             cache.update(B=B, t=(f(B, 2), f(B, 4, N + 1), f(B, 2, N), i(B), i(B), f(B), f(B), i(B, 4)))
         return BatchResult(*(t.numpy() for t in cache["t"]))
 
-    def _solve_batch_device(self, x0, ref, u_prev, s, stream) -> BatchResult:
+    def _solve_batch_device(self, x0, ref, u_prev, s, stream, rows=None) -> BatchResult:
         import torch
         N = self._params.horizon
         B = x0.shape[0]
@@ -280,6 +340,15 @@ class MPCController:
         h = self._handle(B)
         st = stream if stream is not None else torch.cuda.current_stream(dev).cuda_stream
         p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        if rows is not None:
+            d_par = params_to_device(rows, dev)
+            rc = h.lib.cudampc_solve_batch_params(h.ptr, B, p(x0), p(ref), p(u_prev), C.byref(s), p(d_par), p(out.u0), p(out.Xp),
+                                                  p(out.Up), p(out.status), p(out.iters), p(out.pri_res), p(out.dua_res),
+                                                  p(out.info), C.c_void_p(st))
+            _lib.check(h.lib, h.ptr, rc, "cudampc_solve_batch_params")
+            if stream is not None and d_par is not rows:    # the staged records are freed in the current stream's order
+                torch.cuda.synchronize(dev)
+            return out
         rc = h.lib.cudampc_solve_batch(h.ptr, B, p(x0), p(ref), p(u_prev), C.byref(s), p(out.u0), p(out.Xp), p(out.Up),
                                        p(out.status), p(out.iters), p(out.pri_res), p(out.dua_res), p(out.info),
                                        C.c_void_p(st))
@@ -357,4 +426,4 @@ class MPCController:
         return A, Bm, c
 
 
-__all__ = ["MPCParameters", "SolverSettings", "MPCController", "BatchResult"]
+__all__ = ["MPCParameters", "SolverSettings", "MPCController", "BatchResult", "params_array"]
