@@ -72,18 +72,43 @@ __device__ __forceinline__ void sts_f64_if(bool p, unsigned a, double v) {
 // (tools/microbench/oe_bench.cu).  The loop is branch-free between the two halves: both run the trip count of the longer
 // one, a half that is done keeps computing on in-bounds words of the workspace and stores nothing (predicated).
 #define MPC_ROW_LANES 0x00000fffu
-__device__ __forceinline__ void oe_forward_lanes(int lane, const View& w, const OEView& oe) {
+// What row lane r of a half needs of it (oe_half) in a sweep, as 32-bit shared addresses.  The sweeps take a functor that
+// yields it, called inside the row lanes' region: the register form returns the copy it formed once per block and keeps in
+// registers (keep_lane), the other callers form it there (sweep_lane).
+struct SweepLane {
+  int r, cnt, xs;     // row / column of the lane, steps of its half, bytes between consecutive local rows (+-48)
+  unsigned x0;        // row of local stage 0
+  unsigned xlast;     // element r of the row read at the middle step
+  unsigned g0;        // block of local step 1
+  unsigned xm;        // row of the middle stage
+};
+__device__ __forceinline__ SweepLane sweep_lane(int lane, const View& w, const OEView& oe) {
+  const bool bottom = lane >= 6;
+  const OEHalf h = oe_half(w, oe, bottom);
+  SweepLane s;
+  s.r = bottom ? lane - 6 : lane;
+  s.cnt = h.cnt; s.xs = h.xstep * 8;
+  s.x0 = smem_u32(h.x0); s.xlast = smem_u32(h.xlast) + 8 * s.r; s.g0 = smem_u32(h.g0); s.xm = smem_u32(w.nx(2 * oe.jm));
+  return s;
+}
+__device__ __forceinline__ SweepLane keep_lane(SweepLane s) {
+  s.r = (int)opaque_u32((unsigned)s.r); s.cnt = (int)opaque_u32((unsigned)s.cnt); s.xs = (int)opaque_u32((unsigned)s.xs);
+  s.x0 = opaque_u32(s.x0); s.xlast = opaque_u32(s.xlast); s.g0 = opaque_u32(s.g0); s.xm = opaque_u32(s.xm);
+  return s;
+}
+template <class SL>
+__device__ __forceinline__ void oe_forward_lanes(int lane, SL lane_of, const OEView& oe) {
   if (lane < 12) {
+    const SweepLane sl = lane_of();
     const bool bottom = lane >= 6;
-    const int r = bottom ? lane - 6 : lane;
-    const OEHalf h = oe_half(w, oe, bottom);
-    const int cnt = h.cnt, cmax = oe.jm > oe.nb ? oe.jm : oe.nb;     // uniform trip count
-    const int xs = h.xstep * 8;                                      // bytes between consecutive local rows (+-48)
-    const unsigned xlast = smem_u32(h.xlast) + 8 * r;
-    unsigned xrow = smem_u32(h.x0) + xs;                             // row of local stage i (i = 1)
-    unsigned gp = smem_u32(h.g0) + 48 * r;                           // row r of the block of step i
+    const int r = sl.r;
+    const int cnt = sl.cnt, cmax = oe.jm > oe.nb ? oe.jm : oe.nb;   // uniform trip count
+    const int xs = sl.xs;
+    const unsigned xlast = sl.xlast;
+    unsigned xrow = sl.x0 + xs;                                      // row of local stage i (i = 1)
+    unsigned gp = sl.g0 + 48 * r;                                    // row r of the block of step i
     double a[6], gA[6], gB[6], nbA, nbB, y;
-    lds_row(smem_u32(h.x0), a);                                      // y_0 = b'_0
+    lds_row(sl.x0, a);                                               // y_0 = b'_0
     double ymid = lds_f64(xlast);                                    // the half's term for the middle if it has no step
     lds_row(gp, gA); nbA = lds_f64(cnt == 1 ? xlast : xrow + 8 * r);
     for (int i = 1; i <= cmax; i += 2) {
@@ -104,7 +129,7 @@ __device__ __forceinline__ void oe_forward_lanes(int lane, const View& w, const 
     }
     // middle stage: x_m = S'_m^-1 (top term + bottom term); lanes r and r + 6 hold element r of the two terms
     const double yo = __shfl_sync(MPC_ROW_LANES, ymid, bottom ? lane - 6 : lane + 6);
-    double* mrow = w.nx(2 * oe.jm);
+    double* mrow = static_cast<double*>(__cvta_shared_to_generic(sl.xm));
     if (lane < 6) mrow[r] = ymid + yo;
     __syncwarp(MPC_ROW_LANES);
     double xm = 0.0;
@@ -118,18 +143,18 @@ __device__ __forceinline__ void oe_forward_lanes(int lane, const View& w, const 
   }
   __syncwarp();
 }
-__device__ __forceinline__ void oe_backward_lanes(int lane, const View& w, const OEView& oe) {
+template <class SL>
+__device__ __forceinline__ void oe_backward_lanes(int lane, SL lane_of, const OEView& oe) {
   if (lane < 12) {
-    const bool bottom = lane >= 6;
-    const int c = bottom ? lane - 6 : lane;
-    const OEHalf h = oe_half(w, oe, bottom);
+    const SweepLane sl = lane_of();
+    const int c = sl.r;
     const int cmax = oe.jm > oe.nb ? oe.jm : oe.nb;
-    const int xs = h.xstep * 8;
-    int i = h.cnt - 1;                                               // local stage of this half at the current step (< 0: done)
-    unsigned xrow = smem_u32(h.x0) + xs * i;                         // row of local stage i
-    unsigned gp = smem_u32(h.g0) + 288 * i + 8 * c;                  // column c of the block of step i+1
+    const int xs = sl.xs;
+    int i = sl.cnt - 1;                                              // local stage of this half at the current step (< 0: done)
+    unsigned xrow = sl.x0 + xs * i;                                  // row of local stage i
+    unsigned gp = sl.g0 + 288 * i + 8 * c;                           // column c of the block of step i+1
     double a[6], gA[6], gB[6], zA, zB;
-    lds_row(smem_u32(w.nx(2 * oe.jm)), a);                           // x_m
+    lds_row(sl.xm, a);                                               // x_m
     lds_col(gp, gA); zA = lds_f64(xrow + 8 * c);
     for (int s = 0; s < cmax; s += 2, i -= 2) {
       lds_col(gp - 288, gB); zB = lds_f64(xrow - xs + 8 * c);        // local stage i-1
@@ -276,7 +301,10 @@ __device__ __forceinline__ void reg_block_run(double* base, int N, int fpad, int
 #pragma unroll
   for (int j = 0; j < 5; ++j) T.G[j] = 0.0;
   T.ua = 0.0; T.ud = 0.0;
-  if (on) reg_load<STATE>(w, k, R);
+  const StageAddr a = stage_addr(w, oe, k);
+  const SweepLane sl = keep_lane(sweep_lane(lane, w, oe));
+  const bool diag = ev && on && k != 2 * oe.jm;                   // the middle stage's row is solved by the sweeps
+  if (on) reg_load<STATE>(a.rec, R);
   // One loop for both warp roles: the update and the right-hand side are ONE copy of code shared by the two warps (two
   // loops - one per role - measured slower with early polish: the iteration loop competes for the 32 KB instruction cache
   // with the polish code other resident problems run).
@@ -285,33 +313,33 @@ __device__ __forceinline__ void reg_block_run(double* base, int N, int fpad, int
   for (int i = 0; i < nb; ++i) {
     MPC_BTAG(26);
     if (sweeper) {
-      oe_forward_lanes(lane, w, oe);
+      oe_forward_lanes(lane, [&] { return sl; }, oe);
       MPC_BTAG(20);
-      if (ev && on) oe_diag_stage(w, oe, k);
+      if (diag) oe_diag(a.di.p(), a.x.p());
       __syncwarp();
       MPC_BTAG(21);
-      oe_backward_lanes(lane, w, oe);
+      oe_backward_lanes(lane, [&] { return sl; }, oe);
       MPC_BTAG(22);
     }
     MPC_BAR();                                        // B_a: x~ of the even stages
-    if (!ev && on) reg_expand(w, p, c, oe, k, R, T);
+    if (!ev && on) reg_expand(a, p, c, k, R, T);
     MPC_BAR();                                        // B_b: x~ of the odd stages
     MPC_BTAG(23);
-    if (ev && on) reg_gather_even(w, k, T);
-    if (on) reg_update<STATE>(w, p, c, k, R, T);
+    if (ev && on) reg_gather_even(a, N, k, T);
+    if (on) reg_update<STATE>(a, p, c, k, R, T);
     MPC_BAR();                                        // B_c: (d, G) of every stage
     MPC_BTAG(24);
-    if (on) reg_rhs<STATE>(w, p, c, oe, k, R, T);
+    if (on) reg_rhs<STATE>(a, p, c, k, R, T);
     MPC_BAR();                                        // B_d: t_o
     MPC_BTAG(25);
-    if (ev && on) reg_fixup(w, p, c, k, T);
+    if (ev && on) reg_fixup(a, p, c, k, T);
     if (sweeper) __syncwarp();
   }
 #ifdef MPC_TIMING
   if (sweeper && lane == 0 && tags) for (int q = 0; q < 7; ++q) atomicAdd(&tags[20 + q], (unsigned long long)tacc[q]);
 #endif
   MPC_BAR();
-  if (on) reg_store<STATE>(w, k, R);
+  if (on) reg_store<STATE>(a.rec, R);
   MPC_BAR();
 }
 
@@ -401,11 +429,11 @@ struct GroupExec {
     group_sync();
   }
   __device__ __forceinline__ void oe_forward(const View& w, const OEView& oe) {
-    if (chain_warp()) oe_forward_lanes(lane, w, oe);
+    if (chain_warp()) oe_forward_lanes(lane, [&] { return sweep_lane(lane, w, oe); }, oe);
     group_sync();
   }
   __device__ __forceinline__ void oe_backward(const View& w, const OEView& oe) {
-    if (chain_warp()) oe_backward_lanes(lane, w, oe);
+    if (chain_warp()) oe_backward_lanes(lane, [&] { return sweep_lane(lane, w, oe); }, oe);
     group_sync();
   }
   // ---- pair form of an iteration (mpc_pair.h): one lane per pair of stages, neighbours exchanged through shuffles.

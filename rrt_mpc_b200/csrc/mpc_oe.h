@@ -384,15 +384,19 @@ MPC_HD void oe_middle(const OEView& oe, const double* at, const double* ab, doub
   for (int r = 0; r < 6; ++r) y[r] = at[r] + ab[r];
   for (int r = 0; r < 6; ++r) xm[r] = oe_sym_row(oe.sinv + OE_SYM * oe.jm, r, y);
 }
-// diagonal step of even stage k != middle: z = S'^-1 y, in place
+// diagonal step z = S'^-1 y, in place (s: S'^-1 packed, row: y)
+MPC_HD void oe_diag(const double* s, double* row) {
+  double sv[OE_SYM], y[6], z[6];
+  sym_load(s, sv);
+  row_load(row, y);
+  symv6(sv, y, z);
+  row_store(row, z);
+}
+// diagonal step of even stage k != middle
 MPC_HD void oe_diag_stage(const View& w, const OEView& oe, int k) {
   const int j = k >> 1;
   if (j == oe.jm) return;
-  double sv[OE_SYM], y[6], z[6];
-  sym_load(oe.sinv + OE_SYM * j, sv);
-  row_load(w.nx(k), y);
-  symv6(sv, y, z);
-  row_store(w.nx(k), z);
+  oe_diag(oe.sinv + OE_SYM * j, w.nx(k));
 }
 
 // whole factorisation / solve, sequential (host emulation; the CUDA policy runs the same pieces with lanes over stages)

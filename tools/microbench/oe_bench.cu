@@ -133,7 +133,7 @@ __global__ void bench_var(int N, int F, int reps, long long* cyc, double* sink) 
   long long tf = 0;
   for (int r = 0; r < reps; ++r) {
     long long t0 = clock64();
-    if (VAR == 0) oe_forward_lanes(lane, w, oe); else if (VAR == 1) fwd_shfl6(lane, w, oe); else if (VAR == 3) fwd_shfl6_region(lane, w, oe); else fwd_shfl2(lane, w, oe);
+    if (VAR == 0) oe_forward_lanes(lane, [&] { return sweep_lane(lane, w, oe); }, oe); else if (VAR == 1) fwd_shfl6(lane, w, oe); else if (VAR == 3) fwd_shfl6_region(lane, w, oe); else fwd_shfl2(lane, w, oe);
     __syncwarp();
     tf += clock64() - t0;
     for (int k = lane; k <= N; k += 32) { double* x = w.nx(k); for (int t = 0; t < 6; ++t) x[t] = 1.0 + 0.01 * ((k + t + r) % 9); }
@@ -153,13 +153,13 @@ __global__ void bench(int N, int F, int reps, long long* cyc, double* sink) {
   long long tf = 0, td = 0, tb = 0, tfac = 0;
   for (int r = 0; r < reps; ++r) {
     long long t0 = clock64();
-    oe_forward_lanes(lane, w, oe);
+    oe_forward_lanes(lane, [&] { return sweep_lane(lane, w, oe); }, oe);
     __syncwarp();
     long long t1 = clock64();
     for (int k = 2 * lane; k <= N; k += 64) oe_diag_stage(w, oe, k);
     __syncwarp();
     long long t2 = clock64();
-    oe_backward_lanes(lane, w, oe);
+    oe_backward_lanes(lane, [&] { return sweep_lane(lane, w, oe); }, oe);
     __syncwarp();
     long long t3 = clock64();
     tf += t1 - t0; td += t2 - t1; tb += t3 - t2;
