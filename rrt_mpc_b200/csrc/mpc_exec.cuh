@@ -41,9 +41,8 @@ __device__ __forceinline__ void factor_twisted_lanes(int lane, const View& w, in
 // Sweeps of the odd-even block solve (mpc_oe.h), one lane per ROW of a half: lanes 0..5 the top half, 6..11 the bottom
 // half, one instruction stream.  Called by all 32 lanes of the chain warp (lanes >= 12 only keep the warp converged).
 // Per step and lane: 3 x LDS.128 (block row, requested one step ahead) + 6 fmas + one 64-bit store of its element of the
-// new vector, __syncwarp, 3 x LDS.128 to read the whole vector back.  The loop is branch-free: both halves run the trip
-// count of the longer one, a half that is done keeps computing on in-bounds words of the workspace and stores nothing
-// (predicated), so the warp never diverges inside the dependent chain.  Shared-memory accesses are explicit PTX on 32-bit
+// new vector, __syncwarp, 3 x LDS.128 to read the whole vector back.  Both halves run the same steps (see below), so the
+// warp never diverges inside the dependent chain.  Shared-memory accesses are explicit PTX on 32-bit
 // shared addresses (through generic pointers every access pays an address-space conversion), two register sets, unrolled
 // by two.
 // ------------------------------------------------------------------------------------------------
@@ -62,6 +61,7 @@ __device__ __forceinline__ void lds_col(unsigned a, double* r) {       // six do
   asm volatile("ld.shared.f64 %0, [%1+240];" : "=d"(r[5]) : "r"(a));
 }
 __device__ __forceinline__ double lds_f64(unsigned a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
+__device__ __forceinline__ void sts_f64(unsigned a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory"); }
 __device__ __forceinline__ void sts_f64_if(bool p, unsigned a, double v) {
   asm volatile("{ .reg .pred q; setp.ne.u32 q, %0, 0; @q st.shared.f64 [%1], %2; }" ::"r"((unsigned)p), "r"(a), "d"(v) : "memory");
 }
@@ -69,77 +69,94 @@ __device__ __forceinline__ void sts_f64_if(bool p, unsigned a, double v) {
 // warp barriers and shuffles over the twelve-lane mask.  With all 32 lanes executing the loads (the idle ones on duplicate
 // addresses, to keep the warp converged) every 128-bit load cost the shared-memory pipe 4-5 wavefronts instead of 2: with
 // five chain warps per SM that saturated the pipe - 108 cycles per step alone, 170 with five warps sweeping
-// (tools/microbench/oe_bench.cu).  The loop is branch-free between the two halves: both run the trip count of the longer
-// one, a half that is done keeps computing on in-bounds words of the workspace and stores nothing (predicated).
+// (tools/microbench/oe_bench.cu).
+// Both halves run the same number of steps P = max(jm, 1) (jm >= nb: the top half has the most), in one instruction stream,
+// and a step in the loop is the same for every lane: block row (requested one step ahead), 6-fma tree, unconditional store,
+// warp barrier, read back.  What differs between the halves is settled in the addresses, formed once (sweep_lane):
+//   forward   every half ends with its middle step (the one that reads b'_m or the row of zeros, peeled after the loop).  A
+//             half with one step fewer (`lag`) starts with a step on the row of zeros: block row 0, vector 0, so the tree
+//             returns b'_0[r] to the last bit (-0 * 0 terms; see oe_row_dot) and stores it back into row 0 unchanged.  A half
+//             with no step (N < 4) does the middle step that way and passes on its xlast exactly.
+//   backward a lagging half's last step is local stage -1: its store is the only predicated one, in the peeled last step.
+// An odd number of loop steps runs one step ahead of the loop, so that the last block is always in the same register set.
 #define MPC_ROW_LANES 0x00000fffu
-// What row lane r of a half needs of it (oe_half) in a sweep, as 32-bit shared addresses.  The sweeps take a functor that
+// What row lane r of a half needs of it (oe_half) in the sweeps, as 32-bit shared addresses.  The sweeps take a functor that
 // yields it, called inside the row lanes' region: the register form returns the copy it formed once per block and keeps in
-// registers (keep_lane), the other callers form it there (sweep_lane).
+// registers (keep_lane), the other callers form it there (sweep_lane).  Seven words, as many as the stage record of the
+// iteration can spare (the kernel is at 255 registers): the backward sweep's start follows from the forward's with a few
+// integer instructions per sweep, the row stride, the lane's element, the step count and `lag` share one word.
 struct SweepLane {
-  int r, cnt, xs;     // row / column of the lane, steps of its half, bytes between consecutive local rows (+-48)
-  unsigned x0;        // row of local stage 0
-  unsigned xlast;     // element r of the row read at the middle step
-  unsigned g0;        // block of local step 1
+  unsigned fa, fg;    // forward: vector before step 1 (row 0, or the row of zeros), block row of step 1 (or the row of zeros)
+  unsigned fx, fq;    // forward: row of step 1, block row of step 2
+  unsigned xl;        // forward: element r of the row read at the middle step (b'_m for the top half, zeros for the bottom)
   unsigned xm;        // row of the middle stage
+  unsigned geo;       // bits 0-7: 8 r; bit 8: bottom half (rows 48 bytes apart downwards); bit 9: lag; bits 16-31: P - 1
+  __device__ __forceinline__ int r8() const { return (int)(geo & 0xffu); }
+  __device__ __forceinline__ int xs() const { return (geo & 0x100u) ? -8 * BXS : 8 * BXS; }
+  __device__ __forceinline__ bool lag() const { return (geo & 0x200u) != 0u; }
+  __device__ __forceinline__ int nst() const { return (int)(geo >> 16); }    // steps in the loops of both sweeps
 };
 __device__ __forceinline__ SweepLane sweep_lane(int lane, const View& w, const OEView& oe) {
   const bool bottom = lane >= 6;
   const OEHalf h = oe_half(w, oe, bottom);
+  const int r = bottom ? lane - 6 : lane, P = oe.jm > 1 ? oe.jm : 1;
+  const bool lag = h.cnt < P;
+  const unsigned x0 = smem_u32(h.x0), g0 = smem_u32(h.g0) + 48 * r, z = smem_u32(w.nx_zero());
   SweepLane s;
-  s.r = bottom ? lane - 6 : lane;
-  s.cnt = h.cnt; s.xs = h.xstep * 8;
-  s.x0 = smem_u32(h.x0); s.xlast = smem_u32(h.xlast) + 8 * s.r; s.g0 = smem_u32(h.g0); s.xm = smem_u32(w.nx(2 * oe.jm));
+  s.fa = lag ? z : x0; s.fg = lag ? z : g0;
+  s.fx = lag ? x0 : x0 + 8 * h.xstep; s.fq = lag ? g0 : g0 + 288;
+  s.xl = smem_u32(h.xlast) + 8 * r; s.xm = smem_u32(w.nx(2 * oe.jm));
+  s.geo = 8u * r | (bottom ? 0x100u : 0u) | (lag ? 0x200u : 0u) | (unsigned)(P - 1) << 16;
   return s;
 }
 __device__ __forceinline__ SweepLane keep_lane(SweepLane s) {
-  s.r = (int)opaque_u32((unsigned)s.r); s.cnt = (int)opaque_u32((unsigned)s.cnt); s.xs = (int)opaque_u32((unsigned)s.xs);
-  s.x0 = opaque_u32(s.x0); s.xlast = opaque_u32(s.xlast); s.g0 = opaque_u32(s.g0); s.xm = opaque_u32(s.xm);
+  s.fa = opaque_u32(s.fa); s.fg = opaque_u32(s.fg); s.fx = opaque_u32(s.fx); s.fq = opaque_u32(s.fq);
+  s.xl = opaque_u32(s.xl); s.xm = opaque_u32(s.xm); s.geo = opaque_u32(s.geo);
   return s;
 }
 template <class SL>
 __device__ __forceinline__ void oe_forward_lanes(int lane, SL lane_of, const OEView& oe) {
   if (lane < 12) {
     const SweepLane sl = lane_of();
-    const bool bottom = lane >= 6;
-    const int r = sl.r;
-    const int cnt = sl.cnt, cmax = oe.jm > oe.nb ? oe.jm : oe.nb;   // uniform trip count
-    const int xs = sl.xs;
-    const unsigned xlast = sl.xlast;
-    unsigned xrow = sl.x0 + xs;                                      // row of local stage i (i = 1)
-    unsigned gp = sl.g0 + 48 * r;                                    // row r of the block of step i
+    const int xs = sl.xs(), r8 = sl.r8(), nst = sl.nst();
+    unsigned xrow = sl.fx, gq = sl.fq;                               // row of the current step, block row of the next one
     double a[6], gA[6], gB[6], nbA, nbB, y;
-    lds_row(sl.x0, a);                                               // y_0 = b'_0
-    double ymid = lds_f64(xlast);                                    // the half's term for the middle if it has no step
-    lds_row(gp, gA); nbA = lds_f64(cnt == 1 ? xlast : xrow + 8 * r);
-    for (int i = 1; i <= cmax; i += 2) {
-      lds_row(gp + 288, gB); nbB = lds_f64(i + 1 == cnt ? xlast : xrow + xs + 8 * r);          // step i+1
+    lds_row(sl.fa, a);                                               // y_0 = b'_0
+    lds_row(sl.fg, gA); nbA = lds_f64(xrow + r8);
+    const double nbm = lds_f64(sl.xl);                               // b'_m or 0: not written by the sweep
+    if (nst & 1) {
       y = oe_row_dot(gA, nbA, a);
-      ymid = (i == cnt) ? y : ymid;
-      sts_f64_if(i < cnt, xrow + 8 * r, y);
+      lds_row(gq, gA); nbA = lds_f64(xrow + xs + r8);
+      sts_f64(xrow + r8, y);
       __syncwarp(MPC_ROW_LANES);
       lds_row(xrow, a);
-      if (i + 1 > cmax) break;
-      lds_row(gp + 576, gA); nbA = lds_f64(i + 2 == cnt ? xlast : xrow + 2 * xs + 8 * r);      // step i+2
+      gq += 288; xrow += xs;
+    }
+#pragma unroll 1
+    for (int n = nst >> 1; n > 0; --n) {
+      lds_row(gq, gB); nbB = lds_f64(xrow + xs + r8);
+      y = oe_row_dot(gA, nbA, a);
+      sts_f64(xrow + r8, y);
+      __syncwarp(MPC_ROW_LANES);
+      lds_row(xrow, a);
+      lds_row(gq + 288, gA); nbA = lds_f64(xrow + 2 * xs + r8);    // the middle step reads nbm instead
       y = oe_row_dot(gB, nbB, a);
-      ymid = (i + 1 == cnt) ? y : ymid;
-      sts_f64_if(i + 1 < cnt, xrow + xs + 8 * r, y);
+      sts_f64(xrow + xs + r8, y);
       __syncwarp(MPC_ROW_LANES);
       lds_row(xrow + xs, a);
-      gp += 576; xrow += 2 * xs;
+      gq += 576; xrow += 2 * xs;
     }
-    // middle stage: x_m = S'_m^-1 (top term + bottom term); lanes r and r + 6 hold element r of the two terms
-    const double yo = __shfl_sync(MPC_ROW_LANES, ymid, bottom ? lane - 6 : lane + 6);
-    double* mrow = static_cast<double*>(__cvta_shared_to_generic(sl.xm));
-    if (lane < 6) mrow[r] = ymid + yo;
+    const double ymid = oe_row_dot(gA, nbm, a);                      // the half's term for the middle stage
+    // middle stage: x_m = S'_m^-1 (top term + bottom term).  Lanes r and r + 6 hold element r of the two terms and both
+    // form and store the same sum (addition commutes exactly) and the same row of S'_m^-1 times it: no divergence.
+    const double yo = __shfl_sync(MPC_ROW_LANES, ymid, lane < 6 ? lane + 6 : lane - 6);
+    sts_f64(sl.xm + r8, ymid + yo);
     __syncwarp(MPC_ROW_LANES);
-    double xm = 0.0;
-    if (lane < 6) {
-      double s[6];
-      row_load(mrow, s);
-      xm = oe_sym_row(oe.sinv + OE_SYM * oe.jm, r, s);
-    }
+    double s[6];
+    lds_row(sl.xm, s);
+    const double xm = oe_sym_row(oe.sinv + OE_SYM * oe.jm, r8 >> 3, s);
     __syncwarp(MPC_ROW_LANES);
-    if (lane < 6) mrow[r] = xm;
+    sts_f64(sl.xm + r8, xm);
   }
   __syncwarp();
 }
@@ -147,27 +164,33 @@ template <class SL>
 __device__ __forceinline__ void oe_backward_lanes(int lane, SL lane_of, const OEView& oe) {
   if (lane < 12) {
     const SweepLane sl = lane_of();
-    const int c = sl.r;
-    const int cmax = oe.jm > oe.nb ? oe.jm : oe.nb;
-    const int xs = sl.xs;
-    int i = sl.cnt - 1;                                              // local stage of this half at the current step (< 0: done)
-    unsigned xrow = sl.x0 + xs * i;                                  // row of local stage i
-    unsigned gp = sl.g0 + 288 * i + 8 * c;                           // column c of the block of step i+1
+    const int xs = sl.xs(), c8 = sl.r8(), nst = sl.nst();
+    // row of local stage i and column c of the block of step i+1, at step 1: local stage cnt - 1 of the half
+    unsigned xrow = sl.fx + xs * (nst - 1), gp = sl.fq - 5 * c8 + 288 * (nst - 1);
     double a[6], gA[6], gB[6], zA, zB;
     lds_row(sl.xm, a);                                               // x_m
-    lds_col(gp, gA); zA = lds_f64(xrow + 8 * c);
-    for (int s = 0; s < cmax; s += 2, i -= 2) {
-      lds_col(gp - 288, gB); zB = lds_f64(xrow - xs + 8 * c);        // local stage i-1
-      sts_f64_if(i >= 0, xrow + 8 * c, oe_row_dot(gA, zA, a));
+    lds_col(gp, gA); zA = lds_f64(xrow + c8);
+    if (nst & 1) {
+      const double x = oe_row_dot(gA, zA, a);
+      lds_col(gp - 288, gA); zA = lds_f64(xrow - xs + c8);
+      sts_f64(xrow + c8, x);
       __syncwarp(MPC_ROW_LANES);
       lds_row(xrow, a);
-      if (s + 1 >= cmax) break;
-      lds_col(gp - 576, gA); zA = lds_f64(xrow - 2 * xs + 8 * c);    // local stage i-2
-      sts_f64_if(i - 1 >= 0, xrow - xs + 8 * c, oe_row_dot(gB, zB, a));
+      gp -= 288; xrow -= xs;
+    }
+#pragma unroll 1
+    for (int n = nst >> 1; n > 0; --n) {
+      lds_col(gp - 288, gB); zB = lds_f64(xrow - xs + c8);          // local stage i-1
+      sts_f64(xrow + c8, oe_row_dot(gA, zA, a));
+      __syncwarp(MPC_ROW_LANES);
+      lds_row(xrow, a);
+      lds_col(gp - 576, gA); zA = lds_f64(xrow - 2 * xs + c8);      // local stage i-2
+      sts_f64(xrow - xs + c8, oe_row_dot(gB, zB, a));
       __syncwarp(MPC_ROW_LANES);
       lds_row(xrow - xs, a);
       gp -= 576; xrow -= 2 * xs;
     }
+    sts_f64_if(!sl.lag(), xrow + c8, oe_row_dot(gA, zA, a));       // local stage 0 (-1 for a lagging half: no store)
   }
   __syncwarp();
 }
